@@ -10,11 +10,17 @@ Workload (BASELINE.json configs[1]/[2]): ViT 7 layers / hidden 384 / 12 heads / 
 fp32 accumulation, per-GPU batch 1024 (weak scaling: global batch = 1024 * N; 8192 at N = 8), synthetic
 32x32x3 data.  One "step" = one optimisation step over one batch.
 
-Prints ONE JSON line (rank 0).  `value` = steady-state img/s with the batch resident in HBM; `e2e` = the same
-through the public API from pinned HOST buffers (H2D of every batch and D2H of every loss inside the timed region).
-`--impl reference` times the reference's own modules (oracle/_ref, a verbatim copy made by oracle/make_ref.py where
-/root/reference is mounted; kind "reference") or, without that copy, the CPU restatement (oracle/, kind "port") on the
-host cores over a bounded sample.  `--impl eager` times the same PyTorch modules on the B200 (eager ATen / cuBLAS: fp32
+Prints ONE JSON line (rank 0).  `value` = steady-state img/s with the batch resident in HBM over `--steps` timed steps;
+`e2e` = the same through the public API from pinned HOST buffers (H2D of every batch and D2H of every loss inside the timed
+region); `step_ms` = per-step times of `--steps` more steps.  The side measurements after them have fixed sizes whatever
+`--steps` says: the per-kernel probe (3 eager steps), `cpu_baseline` (3 steps of at most 128 images) and `gpu_eager_baseline`
+(10 steps).  `--dump-outputs DIR` also writes what the last step of the first timed loop returned to its caller (loss, logits,
+updated parameters, gradients) as DIR/<name>.npy in float32; the inputs depend on the arguments only, so two builds can be
+compared output for output.
+`cpu_baseline`, `gpu_eager_baseline`, `--impl reference` and `--impl eager` time the reference's own modules where their
+source is available (VITB_REFERENCE_ROOT, oracle/_ref or baseline/_ref, see oracle/ref_shim.py; kind "reference"), else
+the oracle's restatement of them (oracle/, kind "port").  `--impl reference` runs on the host cores over a bounded sample;
+`--impl eager` times the same PyTorch modules on the B200 (eager ATen / cuBLAS: fp32
 with matmul precision "medium" as main.py:173, bf16 and fp16 autocast as main.py:58, and torch.compile) — the
 kernel-level bar the hand-written kernels have to beat, since the reference ships no GPU code of its own.
 """
@@ -118,7 +124,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------
 def torch_reference_model():
     """(model, criterion, kind): the reference's own vit.ViT + LabelSmoothingCrossEntropyLoss when a copy of the reference is
-    reachable (oracle/_ref on the GPU box, /root/reference in the authoring container; kind "reference"), else the oracle's
+    reachable (VITB_REFERENCE_ROOT, oracle/_ref or baseline/_ref, see oracle/ref_shim.py; kind "reference"), else the oracle's
     restatement with the same state_dict names (kind "port").  Same construction arguments as utils.get_model (utils.py:71-83)."""
     import torch
     import oracle
@@ -448,6 +454,39 @@ def dp_verify(eng, vb, dist, pg, dev, rank, world):
 
 
 # ---------------------------------------------------------------------------------------------
+# --dump-outputs: what one training step returns to its caller, for comparing two builds output for output
+# ---------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20  # all .npy files of one dump together stay below 64 MB, headers included
+
+
+def step_outputs(eng):
+    """Host float32 copies of what the engine's last step hands its caller: the loss, the logits, the updated parameters and the
+    gradients they were updated with (both flattened and concatenated in state_dict order)."""
+    import torch
+    with torch.no_grad():
+        params = torch.cat([t.detach().float().flatten() for t in eng.model.state_dict().values()])
+        grads = torch.cat([g.float().flatten() for g in eng.grads().values()])
+        return {"loss": eng.loss.float().cpu().numpy(), "logits": eng.logits.float().cpu().numpy(),
+                "params": params.cpu().numpy(), "grads": grads.cpu().numpy()}
+
+
+def dump_outputs(outdir, arrays, seed=0):
+    """Writes every array as outdir/<name>.npy.  The smaller arrays are kept whole; an array that does not fit its share of
+    DUMP_BYTES is replaced by its values at a fixed, seeded set of positions (sorted; the same on every run with the same shapes)."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    left = DUMP_BYTES // 4
+    items = sorted(arrays.items(), key=lambda kv: kv[1].size)
+    for i, (name, a) in enumerate(items):
+        a = np.asarray(a, dtype=np.float32)
+        share = left // (len(items) - i)
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(seed).choice(a.size, size=share, replace=False))]
+        np.save(os.path.join(outdir, f"{name}.npy"), a)
+        left -= a.size
+
+
+# ---------------------------------------------------------------------------------------------
 def run_ours(args):
     global eng_numel
     import torch
@@ -514,6 +553,7 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     ms_dev = timed(lambda i: eng.step(), args.steps, W)
+    outputs = step_outputs(eng) if args.dump_outputs and rank == 0 else None  # taken now: the arms below keep training
     # ---- end-to-end arm: pinned host -> device every step, loss read back every step ----------
     # Public API as a training loop uses it: step() on the batch prefetched during the previous step, then prefetch() of the
     # next pinned host batch (its PCIe transfer overlaps this step's kernels).  One H2D batch copy and one D2H loss read per step.
@@ -524,9 +564,9 @@ def run_ours(args):
         loss_host[i % loss_host.numel()].copy_(loss, non_blocking=True)
     ms_e2e = timed(e2e_step, args.steps, W)
     clocks = sampler.stop() if rank == 0 else None
-    # ---- per-step distribution (SURVEY.md §8d: median + p10/p90): one event pair per step, outside the contract's timed regions
+    # ---- per-step distribution (SURVEY.md §8d: median + p10/p90): one event pair per step, outside the two timed regions
     evs = []
-    for i in range(max(args.steps, 20)):
+    for i in range(args.steps):
         s_, e_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s_.record(); eng.step(); e_.record()
         evs.append((s_, e_))
@@ -603,6 +643,8 @@ def run_ours(args):
                 r = kernel_roofline(row, pk, B, model.num_tokens, model.hidden)
                 row["roofline"] = r
             json.dump({"ms_per_step_graph": ms_dev / args.steps, "img_per_s": value, "kernels": table}, open(args.kernel_table, "w"), indent=1)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1 and dp_check is not None and not dp_check["ok"]:
         sys.stdout.flush()
         os._exit(3)  # a data-parallel numeric mismatch is a failed run, not a benchmark line
@@ -629,7 +671,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--kernel-table", default=None, help="write the per-kernel CUDA-event table (JSON) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the loss, logits, parameters and gradients of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     global MODEL, PER_GPU_BATCH
     MODEL, PER_GPU_BATCH = WORKLOADS[args.workload]
     if args.batch is None:

@@ -9,10 +9,10 @@ when its CUDA library is missing.
 
 Parity status: the reference ships no tests or golden vectors (SURVEY.md §4),
 so the oracle is pinned against the reference itself: ``tests/golden/make_golden.py``
-imports the unmodified reference modules from ``/root/reference`` (two import
+imports the unmodified reference modules from a checkout of it (two import
 shims, see ``oracle/ref_shim.py``), runs them in fp32 on CPU and commits the
 outputs as fixtures; ``tests/test_oracle.py`` checks this restatement against
-those fixtures (and against the live reference whenever it is mounted).
+those fixtures (and against the live reference whenever its source is available).
 """
 from .vit_oracle import (  # noqa: F401
     ViTConfig,

@@ -1,13 +1,13 @@
 """Recipe for oracle/_ref: a verbatim copy of the reference's own implementation of the hot path (TEST INFRASTRUCTURE).
 
-    python oracle/make_ref.py            (also run by __graft_entry__.build() whenever /root/reference is mounted)
+    [VITB_REFERENCE_ROOT=<checkout of mahbodnr/ViT-CIFAR>] python oracle/make_ref.py     (also run by __graft_entry__.build())
 
 The reference is pure Python (no build system, nothing to compile): the "build" is a byte-for-byte copy of the modules that
 `import vit` pulls in — vit.py, layers.py, criterions.py and what layers.py imports at module level (autoencoders.py,
-hamburger/, nnmf/) — from where they lie under /root/reference into oracle/_ref/.  That directory is git-ignored (no reference
-source enters the history) but travels to the GPU box with the snapshot, so `bench.py --impl reference` / `--impl eager`
-and the cpu_baseline leg time the reference ITSELF there (kind "reference") instead of the oracle port, and the live-reference
-tests of tests/test_oracle.py can run on the box too.  A manifest with the sha256 of every copied file is written next to them.
+hamburger/, nnmf/) — from the checkout VITB_REFERENCE_ROOT names, else from an installed copy in baseline/_ref/, into
+oracle/_ref/.  That directory is git-ignored (no reference source enters the history); where it exists, `bench.py --impl reference` / `--impl eager` and the cpu_baseline leg time the
+reference ITSELF (kind "reference") instead of the oracle port, and the live-reference tests of tests/test_oracle.py run.
+A manifest with the sha256 of every copied file is written next to them.
 """
 from __future__ import annotations
 
@@ -17,16 +17,16 @@ import os
 import shutil
 import sys
 
-SRC = os.environ.get("VITB_REFERENCE_SRC", "/root/reference")
 DST = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+SRC = os.environ.get("VITB_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.dirname(DST)), "baseline", "_ref")
 FILES = ["vit.py", "layers.py", "criterions.py", "autoencoders.py"]
 PACKAGES = ["hamburger", "nnmf"]
 
 
 def make_ref(verbose: bool = True) -> bool:
-    if not os.path.isfile(os.path.join(SRC, "vit.py")):
+    if os.path.abspath(SRC) == DST or not os.path.isfile(os.path.join(SRC, "vit.py")):
         if verbose:
-            print(f"make_ref: {SRC} not mounted; keeping whatever is in {DST}")
+            print(f"make_ref: no reference source at {SRC}; keeping whatever is in {DST}")
         return False
     os.makedirs(DST, exist_ok=True)
     manifest = {}

@@ -1,9 +1,12 @@
 """Import the UNMODIFIED reference modules (TEST INFRASTRUCTURE).
 
-From /root/reference where it is mounted (the authoring container), else from
-``oracle/_ref`` — the verbatim copy ``oracle/make_ref.py`` makes there, which is
-git-ignored but travels to the GPU box.  Nothing on the GPU box reads
-/root/reference.  Two shims are needed (SURVEY.md §0):
+The first of these that holds the reference's ``vit.py``: the checkout of
+mahbodnr/ViT-CIFAR named by ``VITB_REFERENCE_ROOT``; ``oracle/_ref``, the verbatim
+copy ``oracle/make_ref.py`` makes; ``baseline/_ref``, where an installed copy of the
+reference is placed beside a checkout.  Both directories are git-ignored: the
+reference is not part of this repository.  Without it, the tests that run it live
+skip, and the fixtures under tests/golden/ (its stored outputs) stand in for it.
+Two shims are needed (SURVEY.md §0):
   * vit.py:3 imports ``torchsummary`` (unused, not installed);
   * layers.py:12 -> nnmf/optimizer.py:8 imports the private
     ``torch.optim.optimizer._dispatch_sqrt`` removed in torch 2.11.
@@ -15,10 +18,10 @@ import os
 import sys
 import types
 
-_COPY = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
-REFERENCE_ROOT = os.environ.get("VITB_REFERENCE_ROOT", "/root/reference")
-if not os.path.isfile(os.path.join(REFERENCE_ROOT, "vit.py")) and os.path.isfile(os.path.join(_COPY, "vit.py")):
-    REFERENCE_ROOT = _COPY
+_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+CANDIDATES = [os.path.abspath(p) for p in (os.environ.get("VITB_REFERENCE_ROOT"), os.path.join(_REPO, "oracle", "_ref"), os.path.join(_REPO, "baseline", "_ref")) if p]
+REFERENCE_ROOT = next((p for p in CANDIDATES if os.path.isfile(os.path.join(p, "vit.py"))), CANDIDATES[0])
+SKIP_REASON = "the reference's source is not available (VITB_REFERENCE_ROOT, oracle/_ref or baseline/_ref)"
 
 
 def reference_available() -> bool:
@@ -28,7 +31,7 @@ def reference_available() -> bool:
 def import_reference():
     """Returns (vit, layers, criterions) reference modules."""
     if not reference_available():
-        raise FileNotFoundError(f"reference not mounted at {REFERENCE_ROOT}")
+        raise FileNotFoundError(f"no reference source at {REFERENCE_ROOT}")
     import torch
     import torch.optim.optimizer as opt_mod
 

@@ -1,7 +1,7 @@
 """fp32 CPU restatement of the ViT-CIFAR training step (TEST INFRASTRUCTURE).
 
-Every function cites the reference lines it follows (paths relative to
-``/root/reference``).  The arithmetic is plain PyTorch fp32 on CPU, the same
+Every function cites the reference lines it follows (paths relative to the
+root of a mahbodnr/ViT-CIFAR checkout).  The arithmetic is plain PyTorch fp32 on CPU, the same
 library the reference itself computes with (SURVEY.md §8c: all arithmetic on
 this path is ``torch``'s), written functionally over a ``dict`` of tensors that
 uses the reference's ``state_dict`` names, so that weights interchange with the
@@ -368,7 +368,7 @@ def train_step(params: Params, x: torch.Tensor, y: torch.Tensor, cfg: ViTConfig,
 
 # ---------------------------------------------------------------------------
 # nn.Module wrapper (same state_dict names as vit.ViT) — used as the timed CPU
-# baseline ("port") where /root/reference is not mounted (the GPU box).
+# baseline ("port") where the reference's source is not available (oracle/ref_shim.py).
 # ---------------------------------------------------------------------------
 
 class OracleViT(nn.Module):

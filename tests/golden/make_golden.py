@@ -1,9 +1,9 @@
-"""Generate golden fixtures from the UNMODIFIED reference (run in the authoring container only).
+"""Generate golden fixtures from the UNMODIFIED reference.
 
-    python tests/golden/make_golden.py
+    VITB_REFERENCE_ROOT=<checkout of mahbodnr/ViT-CIFAR> python tests/golden/make_golden.py
 
 Imports ``vit.ViT`` / ``criterions.LabelSmoothingCrossEntropyLoss`` from
-/root/reference (via oracle/ref_shim.py), loads hash-derived weights and inputs
+that checkout (via oracle/ref_shim.py), loads hash-derived weights and inputs
 (oracle.hash_init_ / oracle.hash_inputs: integer arithmetic, reproducible bit for
 bit anywhere), runs forward + LS-CE + backward + torch.optim.Adam (the optimiser
 network.py:71-77 configures) in fp32 on CPU and stores the results.
@@ -128,9 +128,115 @@ def dropout_block():
     print(f"dropout_block: keep rates {[round(m.float().mean().item(), 3) for m in masks.values()]} -> {path} ({os.path.getsize(path) / 1e6:.2f} MB)")
 
 
+# the configurations of tests/test_oracle.py::test_oracle_matches_live_reference
+SEEDED = {
+    "seeded_cls": dict(num_classes=10, img_size=32, patch=8, num_layers=2, hidden=64, mlp_hidden=96, head=4),
+    "seeded_nocls": dict(num_classes=100, img_size=32, patch=4, num_layers=1, hidden=64, mlp_hidden=64, head=2, is_cls_token=False),
+}
+# the model of tests/test_host_logic.py::test_checkpoint_format_round_trip
+CHECKPOINT_KW = dict(img_size=32, patch=4, num_layers=2, hidden=128, mlp_hidden=128, head=4)
+
+
+def seeded_reference():
+    """The reference's OWN initialisation (torch.manual_seed(2045), main.py:150) and one LS-CE forward + backward on torch.randn
+    inputs drawn right after it, for the two configurations the live comparison uses; plus the state_dict names and shapes of
+    the checkpoint test's model.  Same draws, in the same order, as the live tests."""
+    ref_vit, _, ref_crit = import_reference()
+    torch.set_num_threads(1)
+    for name, kw in SEEDED.items():
+        cfg = ViTConfig(**kw)
+        torch.manual_seed(2045)
+        model = ref_vit.ViT(3, cfg.num_classes, img_size=cfg.img_size, patch=cfg.patch, num_layers=cfg.num_layers,
+                            hidden=cfg.hidden, mlp_hidden=cfg.mlp_hidden, head=cfg.head, is_cls_token=cfg.is_cls_token)
+        state_dict = {k: v.detach().clone() for k, v in model.state_dict().items()}
+        x = torch.randn(3, 3, 32, 32)
+        y = torch.randint(0, cfg.num_classes, (3,))
+        logits = model(x)
+        loss = ref_crit.LabelSmoothingCrossEntropyLoss(cfg.num_classes, 0.1)(logits, y)
+        loss.backward()
+        out = dict(cfg=kw, state_dict=state_dict, x=x, y=y, logits=logits.detach().clone(), loss=loss.item(),
+                   grads={k: p.grad.detach().clone() for k, p in model.named_parameters()}, torch_version=torch.__version__)
+        if name == "seeded_cls":
+            out["checkpoint_shapes"] = {k: tuple(v.shape) for k, v in ref_vit.ViT(3, 10, **CHECKPOINT_KW).state_dict().items()}
+        _save(out, name)
+
+
+def dropout_sites():
+    """The reference block in training mode at p = 0.3 with and without its MLP (layers.py:35, 38, 102), as the live test
+    builds it: the masks torch drew (forward hooks), the output, every gradient for a random cotangent, and the eval output."""
+    _, ref_layers, _ = import_reference()
+    torch.set_num_threads(1)
+    out = {}
+    for use_mlp in (True, False):
+        p_drop = 0.3
+        torch.manual_seed(11)
+        blk = ref_layers.TransformerEncoder(64, 96, head=4, dropout=p_drop, use_mlp=use_mlp)
+        blk.train()
+        x = torch.randn(3, 17, 64, requires_grad=True)
+        masks = {}
+        sites = {blk.attention.dropout: 0}
+        if use_mlp:
+            sites[blk.mlp[2]] = 1
+            sites[blk.mlp[5]] = 2
+        hooks = [m.register_forward_hook(lambda mod, inp, o, s=s: masks.__setitem__(s, ((o != 0) | (inp[0] == 0)).clone()))
+                 for m, s in sites.items()]
+        y = blk(x)
+        for h in hooks:
+            h.remove()
+        w = torch.randn_like(y)
+        (y * w).sum().backward()
+        blk.eval()
+        out[use_mlp] = dict(p=p_drop, head=4, state_dict={k: v.detach().clone() for k, v in blk.state_dict().items()},
+                            x=x.detach().clone(), w=w, masks=masks, y=y.detach().clone(), dx=x.grad.clone(),
+                            grads={k: (v.grad.detach().clone() if v.grad is not None else None) for k, v in blk.named_parameters()},
+                            y_eval=blk(x.detach()).detach().clone())
+    _save(dict(cases=out, torch_version=torch.__version__), "dropout_sites")
+
+
+def batch_mixing():
+    """da.CutMix(32, 1.0) and da.MixUp(0.1) (da.py:51-93) on a seeded 4-image batch for seeds 0..5, and the reference
+    criterion's two-target loss (network.py:163-165) on seeded logits."""
+    import numpy as np
+    _, _, ref_crit = import_reference()
+    import da as ref_da  # the reference's module (sys.path set by import_reference)
+    g = torch.Generator().manual_seed(3)
+    img = torch.randn(4, 3, 32, 32, generator=g)
+    label = torch.randint(0, 10, (4,), generator=g)
+    cutmix, mixup = [], []
+    for seed in range(6):
+        np.random.seed(seed); torch.manual_seed(seed)
+        o, la, lb, lam = ref_da.CutMix(32, 1.0)((img.clone(), label.clone()))
+        cutmix.append(dict(out=o, label=la, rand_label=lb, lam=lam))
+        np.random.seed(seed); torch.manual_seed(seed)
+        o, la, lb, lam = ref_da.MixUp(0.1)((img, label))
+        mixup.append(dict(out=o, label=la, rand_label=lb, lam=lam))
+    g = torch.Generator().manual_seed(7)
+    z = torch.randn(9, 10, generator=g); ya = torch.randint(0, 10, (9,), generator=g); yb = torch.randint(0, 10, (9,), generator=g)
+    crit = ref_crit.LabelSmoothingCrossEntropyLoss(10, smoothing=0.1)
+    two_target = (crit(z, ya) * 0.37 + crit(z, yb) * (1 - 0.37)).item()
+    _save(dict(img=img, label=label, cutmix=cutmix, mixup=mixup, two_target_loss=two_target, torch_version=torch.__version__),
+          "batch_mixing")
+
+
+def _save(obj, name):
+    path = os.path.join(HERE, f"{name}.pt")
+    torch.save(obj, path)
+    size = os.path.getsize(path)
+    assert size < 1_000_000, (path, size)
+    print(f"{name} -> {path} ({size / 1e6:.2f} MB)")
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "dropout":  # only the newer fixture; the others stay byte-identical
+    which = sys.argv[1] if len(sys.argv) > 1 else "all"
+    if which == "dropout":  # only the newer fixture; the others stay byte-identical
         dropout_block()
+    elif which == "seeded":  # the fixtures of the live-reference tests only
+        seeded_reference()
+        dropout_sites()
+        batch_mixing()
     else:
         main()
         dropout_block()
+        seeded_reference()
+        dropout_sites()
+        batch_mixing()

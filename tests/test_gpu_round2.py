@@ -530,3 +530,45 @@ def test_engine_fused_and_unfused_backward_chains_agree(vb, monkeypatch, p_drop)
         for i in range(cfg.num_layers - 1):  # b2 of every block but the last comes from another kernel's partial sums
             layout.view(diff, f"enc.{i}.mlp.3.bias").fill_(False)
         assert not bool(diff.any())
+
+
+# ---------------------------------------------------------------------------------------------
+# (h) bench.py --dump-outputs: what the last timed step returned, from inputs fixed by the arguments
+# ---------------------------------------------------------------------------------------------
+def test_bench_dumps_the_outputs_of_its_last_timed_step(tmp_path):
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    B, names = 128, ("loss", "logits", "params", "grads")
+
+    def bench(steps, outdir):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", "1", "--batch", str(B),
+                            "--no-cpu-baseline", "--dump-outputs", str(outdir)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert d["steps"] == steps and d["step_ms"]["n"] == steps
+        assert sorted(os.listdir(outdir)) == sorted(f"{n}.npy" for n in names)
+        assert sum(os.path.getsize(outdir / f"{n}.npy") for n in names) <= 64_000_000
+        return {n: np.load(outdir / f"{n}.npy") for n in names}
+
+    out = bench(3, tmp_path / "a")
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in out.values())
+    assert out["loss"].shape == () and out["logits"].shape == (B, 10)
+    assert out["params"].shape == out["grads"].shape == (6_268_810,) and out["grads"].any()
+    # the device-resident loop trains on bench.py's first host batch (torch.Generator seeded 1234: four image batches, then labels)
+    g = torch.Generator().manual_seed(1234)
+    for _ in range(4):
+        torch.randn(B, 3, 32, 32, generator=g)
+    y = torch.randint(0, 10, (B,), generator=g)
+    loss = oracle.ls_ce_loss(torch.from_numpy(out["logits"]).double(), y, 10, 0.1).item()
+    assert abs(float(out["loss"]) - loss) < 1e-4 * abs(loss)
+    # same arguments, same outputs; one more timed step, other parameters (the capture point follows --steps)
+    again = bench(3, tmp_path / "b")
+    for n in names:
+        np.testing.assert_array_equal(again[n], out[n], err_msg=n)
+    later = bench(4, tmp_path / "c")
+    assert not np.allclose(later["params"], out["params"], rtol=0, atol=1e-7)
+    assert float(later["loss"]) != float(out["loss"])

@@ -10,7 +10,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import oracle
-from oracle.ref_shim import import_reference, reference_available
+from oracle.ref_shim import SKIP_REASON, import_reference, reference_available
 
 README = dict(num_classes=10, img_size=32, patch=8, num_layers=7, hidden=384, mlp_hidden=384, head=12)
 
@@ -39,7 +39,7 @@ def test_constructor_signature_and_state_dict_match_oracle_names():
         make(img_size=32, patch=5)  # vit.py:40
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 def test_same_seed_gives_reference_initialisation_and_interchangeable_state_dict():
     ref_vit, _, _ = import_reference()
     kw = dict(img_size=32, patch=4, num_layers=2, hidden=128, mlp_hidden=256, head=4)
@@ -324,7 +324,7 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["impl"] == "reference" and d["unit"] == "img/s" and d["higher_is_better"] is True and d["value"] > 0
     for k in ("metric", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert k in d, k
-    # "reference" when a copy of the reference's own modules is reachable (/root/reference here, oracle/_ref on the GPU box), else the port
+    # "reference" when a copy of the reference's own modules is reachable (VITB_REFERENCE_ROOT or oracle/_ref), else the port
     from oracle import ref_shim
     assert d["cpu_baseline"]["kind"] == ("reference" if ref_shim.reference_available() else "port")
     assert d["cpu_baseline"]["cores"] >= 1 and "sample" in d["cpu_baseline"]
@@ -399,3 +399,25 @@ def test_committed_evidence_lines_carry_the_bench_contract():
         bad = {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
         assert not bad & set(d["clocks"]["reasons"]), (f, d["clocks"])
         assert d["step_ms"]["p10"] <= d["step_ms"]["p50"] <= d["step_ms"]["p90"]
+
+
+def test_bench_output_dump_fits_its_budget_with_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole, large ones as the values at seeded positions that are the same on
+    every run, and the files together stay below 64 MB."""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {"loss": np.float32(2.5), "logits": rng.standard_normal((1024, 10)),
+              "params": rng.standard_normal(12_000_000, dtype=np.float32), "grads": rng.standard_normal(12_000_000, dtype=np.float32)}
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    sizes = 0
+    for name, a in arrays.items():
+        got, again = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, again)
+        sizes += os.path.getsize(tmp_path / "a" / f"{name}.npy")
+        if name in ("loss", "logits"):
+            assert np.array_equal(got, np.asarray(a, dtype=np.float32))
+        else:
+            assert 0 < got.size < a.size and np.isin(got, a).all()
+    assert 50_000_000 < sizes <= 64_000_000

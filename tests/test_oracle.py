@@ -1,5 +1,5 @@
 """CPU: pin the oracle restatement against the fixtures generated from the unmodified reference
-(tests/golden/make_golden.py) and, where /root/reference is mounted, against the live reference."""
+(tests/golden/make_golden.py) and, where the reference's source is available, against the live reference."""
 import math
 import os
 
@@ -8,7 +8,7 @@ import torch
 
 import oracle
 from oracle import ViTConfig
-from oracle.ref_shim import reference_available, import_reference
+from oracle.ref_shim import SKIP_REASON, import_reference, reference_available
 
 FULL = ["tiny65", "tiny17c100", "nocls_nomlp"]
 SUMMARY = ["full65", "full17c100"]
@@ -115,7 +115,7 @@ def test_adam_restatement_matches_torch_adam():
         torch.testing.assert_close(ours[k], p.detach(), rtol=1e-6, atol=1e-7)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 @pytest.mark.parametrize("kw", [
     dict(num_classes=10, img_size=32, patch=8, num_layers=2, hidden=64, mlp_hidden=96, head=4),
     dict(num_classes=100, img_size=32, patch=4, num_layers=1, hidden=64, mlp_hidden=64, head=2, is_cls_token=False),
@@ -185,7 +185,7 @@ def test_philox_restatement_known_answers():
     assert oracle.dropout_threshold(0.0) == 0 and oracle.dropout_keep_mask(64, 0.0, 1, 0, 0).all()
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 @pytest.mark.parametrize("use_mlp", [True, False])
 def test_oracle_dropout_sites_match_live_reference(use_mlp):
     """The three nn.Dropout sites of the reference block (layers.py:35, 38, 102) in training mode: replay the masks torch drew
@@ -260,7 +260,7 @@ def test_sgd_restatement_matches_torch_sgd():
         torch.testing.assert_close(ours[k], p.detach(), rtol=1e-6, atol=1e-7)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 def test_cutmix_mixup_restatements_match_live_reference():
     """da.CutMix / da.MixUp (da.py:51-93) with seeded generators vs the oracle's paste / blend and the product's host-side box
     arithmetic (vit_cifar_b200.cutmix_box draws nothing itself: same numbers in, same box out)."""
