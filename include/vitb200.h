@@ -139,6 +139,16 @@ int vitb_colsum(const void* x, float* colsum, void* ws, size_t ws_bytes, int row
 int vitb_augment_crop_flip_normalize(const uint8_t* img_u8, const int32_t* dx, const int32_t* dy, const uint8_t* flip,
                                      const float* mean3, const float* std3, float* out, int B, int S, int pad, void* stream);
 
+/* AutoAugment sub-policies (the reference's autoaugment.py) fused with RandomCrop + flip + ToTensor + Normalize.
+ * code int32 (B): bits 0-7 sub-policy index, bit 8/9 apply op 1/2, bit 10/11 negative sign of op 1/2 (the caller draws them).
+ * op_ids int32 / mags double: 2*n_sub HOST entries (op code, raw reference magnitude); baked into the launch, graph-capturable.
+ * Op codes: 0 shearX, 1 shearY, 2 translateX, 3 translateY, 4 rotate, 5 color, 6 posterize, 7 solarize, 8 contrast, 9 sharpness,
+ * 10 brightness, 11 autocontrast, 12 equalize, 13 invert.  1 <= n_sub <= 32, S <= 64; other arguments as in
+ * vitb_augment_crop_flip_normalize (dx, dy, flip may be NULL).  An image whose code indexes past the table is written as NaN. */
+int vitb_augment_autoaugment(const uint8_t* img_u8, const int32_t* dx, const int32_t* dy, const uint8_t* flip, const int32_t* code,
+                             const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3,
+                             float* out, int B, int S, int pad, void* stream);
+
 /* ---- batch-level CutMix / MixUp (da.py:51-93; network.py:149-158) on a normalised fp32 (B, C, S, S) device batch; perm int32 (B) =
  * the shuffled partner of every image (the caller draws it, with lam and the box, like the reference does on the host).
  * mode 0: out[b, :, i, j] = img[perm[b], :, i, j] inside rows x1 <= i < x2, columns y1 <= j < y2 (the reference's own index order,

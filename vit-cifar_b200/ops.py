@@ -232,6 +232,23 @@ def augment(img_u8, dx, dy, flip, mean, std, out, pad: int) -> None:
                                                        _ptr(out), B, S, int(pad), _stream()), "augment_crop_flip_normalize")
 
 
+def augment_autoaugment(img_u8, dx, dy, flip, code, op_ids, mags, mean, std, out, pad: int) -> None:
+    """`augment` with an AutoAugment sub-policy (the reference's autoaugment.py) applied between the flip and ToTensor.  code (int32,
+    device): per image, bits 0-7 sub-policy index, 8/9 apply op 1/2, 10/11 negative sign of op 1/2; op_ids / mags: the table, two
+    (op code, magnitude) entries per sub-policy (autoaugment.kernel_table)."""
+    B, S = img_u8.shape[0], img_u8.shape[1]
+    assert img_u8.dtype == torch.uint8 and img_u8.shape == (B, S, S, 3) and out.dtype == torch.float32 and out.shape == (B, 3, S, S)
+    assert (dx is None or dx.dtype == torch.int32) and (dy is None or dy.dtype == torch.int32) and (flip is None or flip.dtype == torch.uint8)
+    assert code.dtype == torch.int32 and code.shape == (B,) and len(op_ids) == len(mags) and len(op_ids) % 2 == 0
+    _contig(img_u8, out, dx, dy, flip, code)
+    m, s_ = _F3(*[float(v) for v in mean]), _F3(*[float(v) for v in std])
+    n = len(op_ids)
+    ids, mg = (C.c_int32 * n)(*[int(v) for v in op_ids]), (C.c_double * n)(*[float(v) for v in mags])
+    check(_lib.load().vitb_augment_autoaugment(_ptr(img_u8), _ptr(dx), _ptr(dy), _ptr(flip), _ptr(code), C.cast(ids, C.c_void_p), C.cast(mg, C.c_void_p),
+                                               n // 2, C.cast(m, C.c_void_p), C.cast(s_, C.c_void_p), _ptr(out), B, S, int(pad), _stream()),
+          "augment_autoaugment")
+
+
 def batch_mix(img, perm, out, mode: int, lam: float = 1.0, box=(0, 0, 0, 0)) -> None:
     """CutMix (mode 0: paste rows box[0]:box[1], columns box[2]:box[3] of img[perm[b]] into img[b], da.py:68) or MixUp (mode 1:
     lam * img + (1 - lam) * img[perm], da.py:90) of an fp32 (B, C, S, S) batch into `out`."""

@@ -90,31 +90,59 @@ CIFAR100_MEAN, CIFAR100_STD = (0.5071, 0.4867, 0.4408), (0.2675, 0.2565, 0.2761)
 
 
 class GpuAugment:
-    """RandomCrop(size, padding) + RandomHorizontalFlip + ToTensor + Normalize(mean, std) — get_transform's training pipeline
-    without AutoAugment — on a raw uint8 (B, S, S, 3) batch that is already on the device: one gather kernel instead of a
-    per-image PIL pipeline in DataLoader workers, and 4x fewer bytes over PCIe than normalised fp32 batches.
-    The random draws use a torch.Generator on the device (torchvision draws them on the host, per image)."""
+    """get_transform's training pipeline — RandomCrop(size, padding) + RandomHorizontalFlip + [AutoAugment policy] + ToTensor +
+    Normalize(mean, std) — on a raw uint8 (B, S, S, 3) batch that is already on the device: one kernel instead of a per-image PIL
+    pipeline in DataLoader workers, and 4x fewer bytes over PCIe than normalised fp32 batches.
+    The random draws use a torch.Generator on the device (torchvision and the reference draw them on the host, per image).
+
+    policy: None (no AutoAugment), "cifar10" (CIFAR10Policy, which the reference also uses for CIFAR-100) or "svhn" (SVHNPolicy);
+    the reference's recipes are
+        c10 / c100   GpuAugment(32, 4, mean, std, policy="cifar10")
+        svhn         GpuAugment(32, 4, mean, std, flip=False, policy="svhn")
+    With a policy, each image also draws its sub-policy (uniform), the two gates (rand < p) and two signs (+-1, p = 1/2) after the
+    crop and flip draws; every op reproduces the Pillow call of the reference's autoaugment.py (csrc/augment.cu).  The draws follow
+    the reference's distribution, not Python's `random` stream."""
 
     def __init__(self, size: int = 32, padding: int = 4, mean=CIFAR10_MEAN, std=CIFAR10_STD, flip: bool = True, seed: int = 0,
-                 device="cuda"):
+                 device="cuda", policy: Optional[str] = None):
         self.size, self.padding, self.mean, self.std, self.flip = int(size), int(padding), tuple(mean), tuple(std), bool(flip)
         self.gen = torch.Generator(device=device)
         self.gen.manual_seed(seed)
+        self.policy = policy
+        if policy is not None:
+            from .autoaugment import POLICIES, kernel_table
+            if policy not in POLICIES:
+                raise ValueError(f"policy must be None or one of {sorted(POLICIES)}, got {policy!r}")
+            self.op_ids, self.mags, probs = kernel_table(policy)
+            self.n_sub = len(self.op_ids) // 2
+            self.probs = torch.tensor(probs, dtype=torch.float64, device=device).view(self.n_sub, 2)
 
     def draw(self, B: int, device):
+        """(dx, dy, flip) without a policy; (dx, dy, flip, code) with one (code as vitb_augment_autoaugment reads it)."""
         hi = 2 * self.padding + 1
         dx = torch.randint(0, hi, (B,), generator=self.gen, device=device, dtype=torch.int32)
         dy = torch.randint(0, hi, (B,), generator=self.gen, device=device, dtype=torch.int32)
         fl = (torch.rand((B,), generator=self.gen, device=device) < 0.5).to(torch.uint8) if self.flip else None  # p = 0.5
-        return dx, dy, fl
+        if self.policy is None:
+            return dx, dy, fl
+        sub = torch.randint(0, self.n_sub, (B,), generator=self.gen, device=device, dtype=torch.int32)
+        gate = torch.rand((B, 2), generator=self.gen, device=device, dtype=torch.float64) < self.probs[sub.long()]
+        neg = torch.rand((B, 2), generator=self.gen, device=device) < 0.5
+        g, s = gate.to(torch.int32), neg.to(torch.int32)
+        code = sub | (g[:, 0] << 8) | (g[:, 1] << 9) | (s[:, 0] << 10) | (s[:, 1] << 11)
+        return dx, dy, fl, code
 
     def __call__(self, img_u8: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         from . import ops
         B = img_u8.shape[0]
         if out is None:
             out = torch.empty((B, 3, self.size, self.size), dtype=torch.float32, device=img_u8.device)
-        dx, dy, fl = self.draw(B, img_u8.device)
-        ops.augment(img_u8, dx, dy, fl, self.mean, self.std, out, self.padding)
+        if self.policy is None:
+            dx, dy, fl = self.draw(B, img_u8.device)
+            ops.augment(img_u8, dx, dy, fl, self.mean, self.std, out, self.padding)
+        else:
+            dx, dy, fl, code = self.draw(B, img_u8.device)
+            ops.augment_autoaugment(img_u8, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, self.padding)
         return out
 
 
