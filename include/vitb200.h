@@ -236,6 +236,18 @@ int vitb_ls_ce_blocks_fwd_bwd(const float* logits, const int64_t* labels_a, cons
                               const float* lam_dev, const int* n_valid_dev, float* loss, float* dlogits, int B, int C,
                               float smoothing, float grad_scale, void* ws, size_t ws_bytes, void* stream);
 
+/* ---- validation metrics of one batch (network.py:388-395): logits fp32 (B,C), labels int64 (B), n_valid_dev device int (NULL = B):
+ * rows >= n_valid are ignored.  totals: 3 device doubles [loss_sum, correct, count], ADDED to (not overwritten), so that one record
+ * accumulates a whole validation pass.  loss per row = the label-smoothing CE of criterions.py:13-19 with `smoothing` (the value
+ * the loss kernels above average); correct = (argmax_j logits[i,j] == label[i]), argmax as torch: the first index of the maximum,
+ * NaN above any number.  A label outside [0, C) is never read through: its row is not correct and adds NaN to loss_sum.
+ * Any C >= 2.  Per-block partial sums in fp64, added in block order: two identical calls give bit-identical totals.
+ * ws: vitb_eval_metrics_ws_bytes() bytes, 8-byte aligned, ZERO before the first call and left zeroed (self-resetting counter;
+ * reusable by the next call on the same stream, not by concurrent calls). ---- */
+size_t vitb_eval_metrics_ws_bytes(void);
+int vitb_eval_metrics(const float* logits, const int64_t* labels, const int* n_valid_dev, int B, int C,
+                      float smoothing, double* totals, void* ws, size_t ws_bytes, void* stream);
+
 /* ---- backward of one nn.Linear y = x W^T (W: [N, K] bf16) in a single pass over dY — what autograd runs as two GEMMs
  * (layers.py:33-37, 85, 102):  dx [M, K] = dy [M, N] W  (times gelu'(z) when z [M, K] != NULL: the Linear's input was GELU(z),
  * layers.py:34);  dw [N, K] fp32 = dy^T x;  dx_colsum [K] fp32 (may be NULL) = column sums of dx as stored, i.e. the bias gradient

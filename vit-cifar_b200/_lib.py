@@ -69,6 +69,8 @@ SIGNATURES = {
     "vitb_ls_ce_batch_fwd_bwd": (_i, [_p, _p, _p, _f, _p, _p, _p, _p, _i, _i, _f, _f, _p]),
     "vitb_ls_ce_ws_bytes": (_sz, []),
     "vitb_ls_ce_blocks_fwd_bwd": (_i, [_p, _p, _p, _f, _p, _p, _p, _p, _i, _i, _f, _f, _p, _sz, _p]),
+    "vitb_eval_metrics_ws_bytes": (_sz, []),
+    "vitb_eval_metrics": (_i, [_p, _p, _p, _i, _i, _f, _p, _p, _sz, _p]),
     "vitb_gemm_bias_act_fwd_drop": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _dp, _p]),
     "vitb_gemm_dgrad_drop": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _dp, _p]),
     "vitb_gelu_bwd_colsum_drop": (_i, [_p, _p, _p, _p, _p, _sz, _i, _i, _i, _dp, _p]),

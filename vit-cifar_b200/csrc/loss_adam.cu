@@ -29,6 +29,16 @@ __device__ __forceinline__ float group_max(float v) {
   return v;
 }
 
+// The per-row arithmetic every loss kernel shares (the training losses and vitb_eval_metrics): from a row's max mx, logit sum sz
+// and sum_j exp(z_j - mx) se, lse = log sum_j exp(z_j) and the smoothed loss sum_j -q_j (z_j - lse) of target logit zy, with
+// q_y = conf = 1 - s and q_j = off = s / (C - 1) elsewhere (criterions.py:13-19)
+__device__ __forceinline__ float ls_ce_lse(float mx, float se) { return mx + logf(se); }
+__device__ __forceinline__ float ls_ce_row_loss(float zy, float sz, float lse, int C, float conf, float off) {
+  return -(conf * (zy - lse) + off * ((sz - zy) - (float)(C - 1) * lse));
+}
+
+// (eval_metrics_kernel walks each row's columns in the same per-lane order, j = lane + G i with i ascending, so that its per-image
+// loss equals the one averaged here for C <= 256: a change of that order here must be made there too)
 // kLsR rows per group and iteration, all their loads (logits, labels) issued before the first reduction: a row is a chain of
 // load -> reduce -> exp -> reduce -> log -> gather z[y] of about two thousand cycles, and a group walks B / (1024 / G) rows
 // (V = logits per lane, R = rows per iteration: 1024 threads leave 64 registers per thread)
@@ -86,11 +96,11 @@ __device__ __forceinline__ float ls_ce_rows(const float* __restrict__ logits, co
         for (int j = gl; j < C; j += G) dlogits[(size_t)r * C + j] = 0.f;
       }
       if (!live[q]) continue;
-      const float lse = mx[q] + logf(se[q]);
+      const float lse = ls_ce_lse(mx[q], se[q]);
       const float zy = logits[(size_t)r * C + y[q]], zb = logits[(size_t)r * C + yb[q]];
-      // sum_j -q_j (z_j - lse) for each target, then the lam mix (criterions.py:13-19 applied twice, network.py:163-165)
-      const float la = -(conf * (zy - lse) + off * ((sz[q] - zy) - (float)(C - 1) * lse));
-      const float lb = -(conf * (zb - lse) + off * ((sz[q] - zb) - (float)(C - 1) * lse));
+      // the loss for each target, then the lam mix (criterions.py:13-19 applied twice, network.py:163-165)
+      const float la = ls_ce_row_loss(zy, sz[q], lse, C, conf, off);
+      const float lb = ls_ce_row_loss(zb, sz[q], lse, C, conf, off);
       if (gl == 0) acc += lam * la + (1.0f - lam) * lb;
       if (dlogits != nullptr) {
 #pragma unroll
@@ -149,10 +159,10 @@ __global__ void __launch_bounds__(1024)
     }
     float se = 0.f;
     for (int j = 0; j < C; ++j) se += expf(z[j] - mx);
-    const float lse = mx + logf(se);
+    const float lse = ls_ce_lse(mx, se);
     const float zy = z[y], zb = z[yb];
-    const float la = -(conf * (zy - lse) + off * ((sz - zy) - (float)(C - 1) * lse));
-    const float lb = -(conf * (zb - lse) + off * ((sz - zb) - (float)(C - 1) * lse));
+    const float la = ls_ce_row_loss(zy, sz, lse, C, conf, off);
+    const float lb = ls_ce_row_loss(zb, sz, lse, C, conf, off);
     acc += lam * la + (1.0f - lam) * lb;
     if (dlogits != nullptr) {
       float* d = dlogits + (size_t)r * C;
@@ -213,6 +223,96 @@ __global__ void __launch_bounds__(kLsBlockThreads)
       float t = 0.f;
       for (unsigned int b = 0; b < gridDim.x; ++b) t += vp[b];
       *loss = t / (float)nv;
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Validation metrics (network.py:388-395): per row the LS-CE loss above and argmax == label, summed over the batch into a
+// [loss_sum, correct, count] record of doubles.  One warp per row, rows gwarp, gwarp + nwarps, ...; a lane walks the columns
+// j = lane + 32 i in increasing i, so any C works, and for C <= 256 a row's max, sum and exp-sum come out bit for bit as in
+// ls_ce_rows (same per-lane order; the xor tree over 32 lanes equals the 16-lane one when lanes 16..31 hold -inf / 0).
+// Per-block partials in fp64, added in block order by the last block to arrive (counter in the first word of ws): deterministic.
+// ---------------------------------------------------------------------------------------------
+constexpr int kEvalThreads = 256;
+constexpr int kEvalMaxBlocks = 256;
+
+// torch.argmax order: NaN above everything, then larger values; equal values -> the smaller index
+__device__ __forceinline__ bool argmax_before(float v, int j, float bv, int bj) {
+  if (isnan(v) != isnan(bv)) return isnan(v);
+  if (isnan(v) || v == bv) return j < bj;
+  return v > bv;
+}
+
+__global__ void __launch_bounds__(kEvalThreads)
+    eval_metrics_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels, const int* __restrict__ n_valid_dev,
+                        int B, int C, float smoothing, double* __restrict__ totals, double* __restrict__ ws) {
+  pdl_trigger();
+  pdl_wait();
+  __shared__ double part[kEvalThreads / 32][2];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const float off = smoothing / (float)(C - 1);
+  const float conf = 1.0f - smoothing;
+  const int nv = n_valid_dev != nullptr ? min(max(*n_valid_dev, 0), B) : B;
+  const int nwarps = (int)gridDim.x * (kEvalThreads / 32);
+  double loss_acc = 0.0, corr_acc = 0.0;  // (lane 0's)
+  for (int r = (int)blockIdx.x * (kEvalThreads / 32) + warp; r < nv; r += nwarps) {
+    const float* z = logits + (size_t)r * C;
+    float mx = -INFINITY, sz = 0.f, bv = -INFINITY;
+    int bj = C;
+    for (int j = lane; j < C; j += 32) {
+      const float v = z[j];
+      mx = fmaxf(mx, v);
+      sz += v;
+      if (argmax_before(v, j, bv, bj)) { bv = v; bj = j; }
+    }
+    mx = group_max<32>(mx);
+    sz = group_sum<32>(sz);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int oj = __shfl_xor_sync(0xffffffffu, bj, o);
+      if (argmax_before(ov, oj, bv, bj)) { bv = ov; bj = oj; }
+    }
+    float se = 0.f;
+    for (int j = lane; j < C; j += 32) se += expf(z[j] - mx);
+    se = group_sum<32>(se);
+    if (lane == 0) {
+      const int64_t y = labels[r];
+      if (y >= 0 && y < C) {  // a label outside [0, C) is never dereferenced: the row is wrong and its loss NaN
+        loss_acc += (double)ls_ce_row_loss(z[y], sz, ls_ce_lse(mx, se), C, conf, off);
+        corr_acc += bj == (int)y ? 1.0 : 0.0;
+      } else {
+        loss_acc += (double)NAN;
+      }
+    }
+  }
+  if (lane == 0) {
+    part[warp][0] = loss_acc;
+    part[warp][1] = corr_acc;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s0 = 0.0, s1 = 0.0;
+    for (int w = 0; w < kEvalThreads / 32; ++w) {
+      s0 += part[w][0];
+      s1 += part[w][1];
+    }
+    volatile double* vp = ws + 1;
+    vp[2 * blockIdx.x] = s0;
+    vp[2 * blockIdx.x + 1] = s1;
+    __threadfence();
+    const unsigned int done = atomicInc(reinterpret_cast<unsigned int*>(ws), gridDim.x - 1);  // wraps to 0 with the last arrival
+    if (done == gridDim.x - 1) {
+      __threadfence();
+      double t0 = 0.0, t1 = 0.0;
+      for (unsigned int b = 0; b < gridDim.x; ++b) {
+        t0 += vp[2 * b];
+        t1 += vp[2 * b + 1];
+      }
+      totals[0] += t0;
+      totals[1] += t1;
+      totals[2] += (double)nv;
     }
   }
 }
@@ -335,6 +435,21 @@ int vitb_ls_ce_blocks_fwd_bwd(const float* logits, const int64_t* labels_a, cons
   if (blocks > kLsMaxBlocks) blocks = kLsMaxBlocks;
   VITB_LAUNCH((ls_ce_blocks_kernel), blocks, kLsBlockThreads, 0, (cudaStream_t)stream, logits, labels_a, labels_b, lam, lam_dev, n_valid_dev, loss, dlogits,
               B, C, smoothing, grad_scale, (float*)ws);
+  VITB_LAUNCH_OK();
+  return 0;
+}
+
+size_t vitb_eval_metrics_ws_bytes(void) { return (size_t)(1 + 2 * kEvalMaxBlocks) * sizeof(double); }
+
+int vitb_eval_metrics(const float* logits, const int64_t* labels, const int* n_valid_dev, int B, int C, float smoothing, double* totals,
+                      void* ws, size_t ws_bytes, void* stream) {
+  VITB_REQUIRE(logits && labels && totals && ws, "eval_metrics: null pointer");
+  VITB_REQUIRE(B > 0 && C > 1, "eval_metrics: bad shape B=%d C=%d", B, C);
+  VITB_REQUIRE(ws_bytes >= vitb_eval_metrics_ws_bytes(), "eval_metrics: workspace too small (%zu < %zu)", ws_bytes, vitb_eval_metrics_ws_bytes());
+  VITB_REQUIRE(((uintptr_t)ws | (uintptr_t)totals) % 8 == 0, "eval_metrics: ws and totals must be 8-byte aligned");
+  int blocks = ceil_div(B, kEvalThreads / 32);
+  if (blocks > kEvalMaxBlocks) blocks = kEvalMaxBlocks;
+  VITB_LAUNCH((eval_metrics_kernel), blocks, kEvalThreads, 0, (cudaStream_t)stream, logits, labels, n_valid_dev, B, C, smoothing, totals, (double*)ws);
   VITB_LAUNCH_OK();
   return 0;
 }

@@ -193,7 +193,9 @@ def mhsa_bwd(dy: torch.Tensor, saved, c: LayerViews, g: LayerViews, dm: Dims, al
 # encoder block: layers.py:44-48
 # ---------------------------------------------------------------------------------------------
 def encoder_fwd(x: torch.Tensor, c: LayerViews, p: LayerViews, dm: Dims, alloc: Alloc, attn_map: Optional[torch.Tensor] = None,
-                drop: Optional[Drop] = None):
+                drop: Optional[Drop] = None, save_preact: bool = True):
+    """`save_preact=False` (forward only, no backward will follow): the two MLP GEMMs do not store their pre-GELU values z1 / z2,
+    which then come back as None in the saved tuple."""
     rows, H, M, act = dm.rows, dm.H, dm.M, x.dtype
     xn = alloc("xn", (rows, H), act)
     mean1 = alloc("mean1", (rows,), torch.float32)
@@ -206,9 +208,9 @@ def encoder_fwd(x: torch.Tensor, c: LayerViews, p: LayerViews, dm: Dims, alloc: 
     mean2 = alloc("mean2", (rows,), torch.float32)
     rstd2 = alloc("rstd2", (rows,), torch.float32)
     ops.layernorm_fwd(x1, H, p.ln2_w, p.ln2_b, x1n, mean2, rstd2, rows, H)
-    z1 = alloc("z1", (rows, M), act)
+    z1 = alloc("z1", (rows, M), act) if save_preact else None
     a1 = alloc("a1", (rows, M), act)
-    z2 = alloc("z2", (rows, H), act)
+    z2 = alloc("z2", (rows, H), act) if save_preact else None
     x2 = alloc("x2", (rows, H), act)
     if drop is not None and _drop_fused(rows):                                     # mlp[0..2]: the mask in the epilogue, after the GELU
         ops.gemm_fwd(x1n, c.w1, p.b1, None, a1, z1, rows, M, H, gelu=True, drop=drop.desc(1))

@@ -333,6 +333,22 @@ def ls_ce_single_block(logits, labels, loss, dlogits, smoothing: float, grad_sca
                                              B, Cn, smoothing, grad_scale, _stream()), "ls_ce_mix_fwd_bwd")
 
 
+def eval_metrics_ws_bytes() -> int:
+    return int(_lib.load().vitb_eval_metrics_ws_bytes())
+
+
+def eval_metrics(logits, labels, totals, ws, smoothing: float, n_valid_dev=None) -> None:
+    """Add the batch's [loss_sum, correct, count] to `totals` (3 float64, device): per row the LS-CE loss of `ls_ce` and
+    argmax == label, over rows [0, n_valid) (`n_valid_dev`: 1-element int32 device tensor, None = all).  `ws`: a zeroed device
+    buffer of eval_metrics_ws_bytes() bytes, reusable by the next call on the same stream."""
+    B, Cn = logits.shape
+    assert logits.dtype == torch.float32 and labels.dtype == torch.int64 and labels.shape == (B,)
+    assert totals.dtype == torch.float64 and totals.numel() == 3 and (n_valid_dev is None or n_valid_dev.dtype == torch.int32)
+    _contig(logits, labels, totals, ws)
+    check(_lib.load().vitb_eval_metrics(_ptr(logits), _ptr(labels), _ptr(n_valid_dev), B, Cn, float(smoothing), _ptr(totals), _ptr(ws),
+                                        ws.numel() * ws.element_size(), _stream()), "eval_metrics")
+
+
 def defer_begin(arena: torch.Tensor) -> None:
     """From here to defer_flush() the second passes of wgrad / LayerNorm-backward / GELU-backward reductions are postponed: their
     partials go into `arena` (uint8 CUDA tensor that must stay alive and untouched until the flush has executed)."""

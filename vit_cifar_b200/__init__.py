@@ -8,6 +8,8 @@ Public surface (mirrors the reference's module/class names for this path):
   LabelSmoothingCrossEntropyLoss                        (criterions.py)
   FusedAdam                                             (torch.optim.Adam as configured in network.py:71-77)
   TrainEngine                                           (the per-batch hot loop, CUDA-graphed, data-parallel)
+  EvalEngine                                            (the validation pass, network.py:388-395: forward-only CUDA graph,
+                                                         loss / accuracy summed on the device, one host sync per pass)
   set_precision / get_precision                         ('bf16' tensor-core path or 'fp32' check mode)
   WarmupCosine, evaluate, save_checkpoint, load_checkpoint   (network.py:113-122, 388-395; main.py:234-237, run_model.py:12-37)
 """
@@ -21,5 +23,6 @@ from .vit import ViT  # noqa: E402,F401
 from .criterions import LabelSmoothingCrossEntropyLoss  # noqa: E402,F401
 from .optim import FusedAdam, adam_hyper, sgd_hyper  # noqa: E402,F401
 from .engine import TrainEngine  # noqa: E402,F401
+from .evaluator import EvalEngine  # noqa: E402,F401
 from .schedule import (WarmupCosine, warmup_cosine_lr, evaluate, save_checkpoint, load_checkpoint, to_lightning_checkpoint,  # noqa: E402,F401
                        GpuAugment, GpuCutMix, GpuMixUp, cutmix_box)
