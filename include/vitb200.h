@@ -149,6 +149,22 @@ int vitb_augment_autoaugment(const uint8_t* img_u8, const int32_t* dx, const int
                              const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3,
                              float* out, int B, int S, int pad, void* stream);
 
+/* ---- the same two transforms reading from a dataset resident in device memory: what the reference's DataLoader does per batch
+ * (RandomSampler / DistributedSampler order, default_collate of the transformed images and their labels; utils.py:452-470 and the
+ * loaders main.py:220-231 passes to Lightning), fused with the transform of utils.py:337-355.
+ * data_u8 uint8 (N,S,S,3) HWC, labels_src int64 (N), idx int32 (B): the dataset row of each batch row (repeats allowed).
+ * Writes out fp32 (B,3,S,S) and labels_dst[b] = labels_src[idx[b]] (int64, B) in the same launch.  For the same draws, out is
+ * bit-identical to vitb_augment_crop_flip_normalize / vitb_augment_autoaugment run on the gathered batch data_u8[idx].  A row
+ * idx[b] outside [0, N) is never dereferenced: that image is written as NaN and its label as -1 (no host round trip).
+ * N >= 1, B >= 1; the policy form takes S <= 64.  Other arguments as in the contiguous forms. ---- */
+int vitb_augment_crop_flip_normalize_gather(const uint8_t* data_u8, const int64_t* labels_src, int N, const int32_t* idx,
+                                            const int32_t* dx, const int32_t* dy, const uint8_t* flip, const float* mean3,
+                                            const float* std3, float* out, int64_t* labels_dst, int B, int S, int pad, void* stream);
+int vitb_augment_autoaugment_gather(const uint8_t* data_u8, const int64_t* labels_src, int N, const int32_t* idx,
+                                    const int32_t* dx, const int32_t* dy, const uint8_t* flip, const int32_t* code,
+                                    const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3,
+                                    float* out, int64_t* labels_dst, int B, int S, int pad, void* stream);
+
 /* ---- batch-level CutMix / MixUp (da.py:51-93; network.py:149-158) on a normalised fp32 (B, C, S, S) device batch; perm int32 (B) =
  * the shuffled partner of every image (the caller draws it, with lam and the box, like the reference does on the host).
  * mode 0: out[b, :, i, j] = img[perm[b], :, i, j] inside rows x1 <= i < x2, columns y1 <= j < y2 (the reference's own index order,
@@ -247,6 +263,11 @@ int vitb_ls_ce_blocks_fwd_bwd(const float* logits, const int64_t* labels_a, cons
 size_t vitb_eval_metrics_ws_bytes(void);
 int vitb_eval_metrics(const float* logits, const int64_t* labels, const int* n_valid_dev, int B, int C,
                       float smoothing, double* totals, void* ws, size_t ws_bytes, void* stream);
+
+/* ---- training-epoch loss record (network.py:206 logs the step loss; the epoch value is its batch-size-weighted mean):
+ * acc[0] += loss[0] * n, in fp64, n = n_valid_dev clamped to [1, B] as the loss kernels do (NULL = B).  loss: the 1-float result of
+ * the loss kernels above; acc: one device double, ADDED to.  One thread; graph-capturable. ---- */
+int vitb_train_loss_accumulate(const float* loss, const int* n_valid_dev, int B, double* acc, void* stream);
 
 /* ---- backward of one nn.Linear y = x W^T (W: [N, K] bf16) in a single pass over dY — what autograd runs as two GEMMs
  * (layers.py:33-37, 85, 102):  dx [M, K] = dy [M, N] W  (times gelu'(z) when z [M, K] != NULL: the Linear's input was GELU(z),

@@ -61,6 +61,8 @@ SIGNATURES = {
     "vitb_pool_bwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _p]),
     "vitb_augment_crop_flip_normalize": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p]),
     "vitb_augment_autoaugment": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i, _i, _i, _p]),
+    "vitb_augment_crop_flip_normalize_gather": (_i, [_p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p]),
+    "vitb_augment_autoaugment_gather": (_i, [_p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _p]),
     "vitb_batch_mix": (_i, [_p, _p, _p, _i, _i, _i, _i, C.c_double, _i, _i, _i, _i, _p]),
     "vitb_dropout_threshold": (C.c_uint32, [_f]),
     "vitb_dropout": (_i, [_p, _p, _p, _i64, _f, C.c_uint64, C.c_uint32, C.c_uint32, _p, _i, _p]),
@@ -71,6 +73,7 @@ SIGNATURES = {
     "vitb_ls_ce_blocks_fwd_bwd": (_i, [_p, _p, _p, _f, _p, _p, _p, _p, _i, _i, _f, _f, _p, _sz, _p]),
     "vitb_eval_metrics_ws_bytes": (_sz, []),
     "vitb_eval_metrics": (_i, [_p, _p, _p, _i, _i, _f, _p, _p, _sz, _p]),
+    "vitb_train_loss_accumulate": (_i, [_p, _p, _i, _p, _p]),
     "vitb_gemm_bias_act_fwd_drop": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _dp, _p]),
     "vitb_gemm_dgrad_drop": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _dp, _p]),
     "vitb_gelu_bwd_colsum_drop": (_i, [_p, _p, _p, _p, _p, _sz, _i, _i, _i, _dp, _p]),

@@ -240,7 +240,8 @@ __device__ void apply_op(const AaEntry& e, bool neg, const uint8_t* in, uint8_t*
 }
 
 __global__ void __launch_bounds__(kAaThreads)
-    augment_autoaugment_kernel(const uint8_t* __restrict__ src, const int32_t* __restrict__ dx, const int32_t* __restrict__ dy,
+    augment_autoaugment_kernel(const uint8_t* __restrict__ src, const int32_t* __restrict__ idx, int N, const int64_t* __restrict__ labels_src,
+                               int64_t* __restrict__ labels_dst, const int32_t* __restrict__ dx, const int32_t* __restrict__ dy,
                                const uint8_t* __restrict__ flip, const int32_t* __restrict__ code, const __grid_constant__ AaTable tab, int n_sub,
                                float m0, float m1, float m2, float s0, float s1, float s2, float* __restrict__ out, int S, int pad) {
   extern __shared__ __align__(16) uint8_t smem[];
@@ -253,11 +254,16 @@ __global__ void __launch_bounds__(kAaThreads)
   pdl_trigger();
   pdl_wait();
 
+  // 0. the source row: image b of the batch, or row idx[b] of a resident N-image dataset (never read outside [0, N): NaN, label -1)
+  const int row = idx ? idx[b] : b;
+  const bool oob = idx != nullptr && (row < 0 || row >= N);
+  if (idx && tid == 0) labels_dst[b] = oob ? -1 : labels_src[row];
+
   // 1. stage: RandomCrop + flip, with augment_kernel's index math (black outside the image)
   const int ox = dx ? dx[b] : pad, oy = dy ? dy[b] : pad;
   const bool fl = flip && flip[b];
-  const uint8_t* img = src + (int64_t)b * NP * 3;
-  for (int p = tid; p < NP; p += blockDim.x) {
+  const uint8_t* img = src + (int64_t)(oob ? 0 : row) * NP * 3;
+  for (int p = oob ? NP : tid; p < NP; p += blockDim.x) {
     const int x = p % S, y = p / S;
     const int sx = (fl ? S - 1 - x : x) + ox - pad, sy = y + oy - pad;
     const bool in = sx >= 0 && sx < S && sy >= 0 && sy < S;
@@ -267,7 +273,7 @@ __global__ void __launch_bounds__(kAaThreads)
 
   // 2. the sub-policy: code bits 0-7 index, 8/9 apply op 1/2, 10/11 negative sign of op 1/2
   const int cd = code[b], sub = cd & 0xff;
-  const bool bad = sub >= n_sub;  // cannot be reported to the host synchronously: the image is written as NaN instead
+  const bool bad = oob || sub >= n_sub;  // cannot be reported to the host synchronously: the image is written as NaN instead
   if (!bad) {
     for (int k = 0; k < 2; ++k) {
       if (!((cd >> (8 + k)) & 1)) continue;
@@ -321,10 +327,10 @@ void rotate_fixed(double deg, int S, int fx[6]) {
 
 using namespace vitb;
 
-int vitb_augment_autoaugment(const uint8_t* img_u8, const int32_t* dx, const int32_t* dy, const uint8_t* flip, const int32_t* code,
-                             const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3, float* out, int B, int S,
-                             int pad, void* stream) {
-  VITB_REQUIRE(img_u8 && code && op_ids && mags && mean3 && std3 && out, "augment_autoaugment: null pointer");
+namespace {
+int launch_autoaugment(const uint8_t* src, const int32_t* idx, int N, const int64_t* labels_src, int64_t* labels_dst, const int32_t* dx,
+                       const int32_t* dy, const uint8_t* flip, const int32_t* code, const int32_t* op_ids, const double* mags, int n_sub,
+                       const float* mean3, const float* std3, float* out, int B, int S, int pad, void* stream) {
   VITB_REQUIRE(B > 0 && S > 0 && S <= kAaMaxS && pad >= 0, "augment_autoaugment: bad shape B=%d S=%d pad=%d (S <= %d)", B, S, pad, kAaMaxS);
   VITB_REQUIRE(n_sub >= 1 && n_sub <= kAaMaxSub, "augment_autoaugment: n_sub=%d outside 1..%d", n_sub, kAaMaxSub);
   VITB_REQUIRE(std3[0] != 0.f && std3[1] != 0.f && std3[2] != 0.f, "augment_autoaugment: zero std");
@@ -340,8 +346,25 @@ int vitb_augment_autoaugment(const uint8_t* img_u8, const int32_t* dx, const int
     tab.e[i].mag = m;
     if (op == AA_ROTATE) rotate_fixed(m, S, tab.e[i].fx);
   }
-  VITB_LAUNCH((augment_autoaugment_kernel), B, kAaThreads, aa_smem_bytes(S), (cudaStream_t)stream, img_u8, dx, dy, flip, code, tab, n_sub, mean3[0],
-              mean3[1], mean3[2], std3[0], std3[1], std3[2], out, S, pad);
+  VITB_LAUNCH((augment_autoaugment_kernel), B, kAaThreads, aa_smem_bytes(S), (cudaStream_t)stream, src, idx, N, labels_src, labels_dst, dx, dy, flip,
+              code, tab, n_sub, mean3[0], mean3[1], mean3[2], std3[0], std3[1], std3[2], out, S, pad);
   VITB_LAUNCH_OK();
   return 0;
+}
+}  // namespace
+
+int vitb_augment_autoaugment(const uint8_t* img_u8, const int32_t* dx, const int32_t* dy, const uint8_t* flip, const int32_t* code,
+                             const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3, float* out, int B, int S,
+                             int pad, void* stream) {
+  VITB_REQUIRE(img_u8 && code && op_ids && mags && mean3 && std3 && out, "augment_autoaugment: null pointer");
+  return launch_autoaugment(img_u8, nullptr, 0, nullptr, nullptr, dx, dy, flip, code, op_ids, mags, n_sub, mean3, std3, out, B, S, pad, stream);
+}
+
+int vitb_augment_autoaugment_gather(const uint8_t* data_u8, const int64_t* labels_src, int N, const int32_t* idx, const int32_t* dx,
+                                    const int32_t* dy, const uint8_t* flip, const int32_t* code, const int32_t* op_ids, const double* mags, int n_sub,
+                                    const float* mean3, const float* std3, float* out, int64_t* labels_dst, int B, int S, int pad, void* stream) {
+  VITB_REQUIRE(data_u8 && labels_src && idx && labels_dst && code && op_ids && mags && mean3 && std3 && out,
+               "augment_autoaugment_gather: null pointer");
+  VITB_REQUIRE(N > 0, "augment_autoaugment_gather: empty dataset (N=%d)", N);
+  return launch_autoaugment(data_u8, idx, N, labels_src, labels_dst, dx, dy, flip, code, op_ids, mags, n_sub, mean3, std3, out, B, S, pad, stream);
 }

@@ -592,27 +592,41 @@ __global__ void pool_bwd_cls_rows_kernel(const T* __restrict__ dy, T* __restrict
 // ---------------------------------------------------------------------------------------------
 // training-time input pipeline on the device (utils.py:337-355): RandomCrop(S, padding) + RandomHorizontalFlip + ToTensor +
 // Normalize as one gather from the raw uint8 HWC batch; the random draws (per-image offsets, flip flags) are inputs.
-//   out[b, c, y, x] = (src(b, y + dy[b] - pad, xs + dx[b] - pad, c) / 255 - mean[c]) / std[c],  xs = flip[b] ? S-1-x : x,
+//   out[b, c, y, x] = (src(r, y + dy[b] - pad, xs + dx[b] - pad, c) / 255 - mean[c]) / std[c],  xs = flip[b] ? S-1-x : x,
 //   src = 0 outside the image (torchvision pads the PIL image with black before ToTensor / Normalize)
+// r = b for a contiguous batch; with idx (the DataLoader's batch assembly, utils.py:452-470) r = idx[b], a row of an N-image
+// resident dataset, and labels_dst[b] = labels_src[r].  A row outside [0, N) is never read: its image is NaN and its label -1.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-    augment_kernel(const uint8_t* __restrict__ src, const int32_t* __restrict__ dx, const int32_t* __restrict__ dy, const uint8_t* __restrict__ flip,
+    augment_kernel(const uint8_t* __restrict__ src, const int32_t* __restrict__ idx, int N, const int64_t* __restrict__ labels_src,
+                   int64_t* __restrict__ labels_dst, const int32_t* __restrict__ dx, const int32_t* __restrict__ dy, const uint8_t* __restrict__ flip,
                    float m0, float m1, float m2, float s0, float s1, float s2, float* __restrict__ out, int B, int S, int pad) {
   pdl_trigger();
   pdl_wait();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x, first = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx)
+    for (int64_t b = first; b < B; b += stride) {
+      const int r = idx[b];
+      labels_dst[b] = (r >= 0 && r < N) ? labels_src[r] : -1;
+    }
   const int64_t total = (int64_t)B * S * S;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t i = first; i < total; i += stride) {
     const int x = (int)(i % S), y = (int)((i / S) % S), b = (int)(i / ((int64_t)S * S));
+    float* o = out + (int64_t)b * 3 * S * S + (int64_t)y * S + x;
+    const int r = idx ? idx[b] : b;
+    if (idx && (r < 0 || r >= N)) {
+      o[0] = o[(int64_t)S * S] = o[(int64_t)2 * S * S] = __int_as_float(0x7fffffff);
+      continue;
+    }
     const int ox = dx ? dx[b] : pad, oy = dy ? dy[b] : pad;
     const int xs = (flip && flip[b]) ? S - 1 - x : x;  // flip acts on the cropped image
     const int sx = xs + ox - pad, sy = y + oy - pad;
-    float r = 0.f, g = 0.f, bl = 0.f;
+    float rr = 0.f, g = 0.f, bl = 0.f;
     if (sx >= 0 && sx < S && sy >= 0 && sy < S) {
-      const uint8_t* p = src + (((int64_t)b * S + sy) * S + sx) * 3;
-      r = (float)p[0] * (1.0f / 255.0f); g = (float)p[1] * (1.0f / 255.0f); bl = (float)p[2] * (1.0f / 255.0f);
+      const uint8_t* p = src + (((int64_t)r * S + sy) * S + sx) * 3;
+      rr = (float)p[0] * (1.0f / 255.0f); g = (float)p[1] * (1.0f / 255.0f); bl = (float)p[2] * (1.0f / 255.0f);
     }
-    float* o = out + (int64_t)b * 3 * S * S + (int64_t)y * S + x;
-    o[0] = (r - m0) / s0;
+    o[0] = (rr - m0) / s0;
     o[(int64_t)S * S] = (g - m1) / s1;
     o[(int64_t)2 * S * S] = (bl - m2) / s2;
   }
@@ -887,8 +901,23 @@ int vitb_augment_crop_flip_normalize(const uint8_t* img_u8, const int32_t* dx, c
   const int64_t total = (int64_t)B * S * S;
   int blocks = (int)ceil_div64(total, 256);
   if (blocks > 16 * kNumSMs) blocks = 16 * kNumSMs;
-  VITB_LAUNCH((augment_kernel), blocks, 256, 0, (cudaStream_t)stream, img_u8, dx, dy, flip, mean3[0], mean3[1], mean3[2], std3[0], std3[1], std3[2], out,
-              B, S, pad);
+  VITB_LAUNCH((augment_kernel), blocks, 256, 0, (cudaStream_t)stream, img_u8, (const int32_t*)nullptr, 0, (const int64_t*)nullptr, (int64_t*)nullptr,
+              dx, dy, flip, mean3[0], mean3[1], mean3[2], std3[0], std3[1], std3[2], out, B, S, pad);
+  VITB_LAUNCH_OK();
+  return 0;
+}
+
+int vitb_augment_crop_flip_normalize_gather(const uint8_t* data_u8, const int64_t* labels_src, int N, const int32_t* idx, const int32_t* dx,
+                                            const int32_t* dy, const uint8_t* flip, const float* mean3, const float* std3, float* out,
+                                            int64_t* labels_dst, int B, int S, int pad, void* stream) {
+  VITB_REQUIRE(data_u8 && labels_src && idx && out && labels_dst && mean3 && std3, "augment_gather: null pointer");
+  VITB_REQUIRE(N > 0 && B > 0 && S > 0 && pad >= 0, "augment_gather: bad shape N=%d B=%d S=%d pad=%d", N, B, S, pad);
+  VITB_REQUIRE(std3[0] != 0.f && std3[1] != 0.f && std3[2] != 0.f, "augment_gather: zero std");
+  const int64_t total = (int64_t)B * S * S;
+  int blocks = (int)ceil_div64(total, 256);
+  if (blocks > 16 * kNumSMs) blocks = 16 * kNumSMs;
+  VITB_LAUNCH((augment_kernel), blocks, 256, 0, (cudaStream_t)stream, data_u8, idx, N, labels_src, labels_dst, dx, dy, flip, mean3[0], mean3[1],
+              mean3[2], std3[0], std3[1], std3[2], out, B, S, pad);
   VITB_LAUNCH_OK();
   return 0;
 }

@@ -454,6 +454,23 @@ int vitb_eval_metrics(const float* logits, const int64_t* labels, const int* n_v
   return 0;
 }
 
+// the epoch record of a training step (network.py:206 logs each step's loss; Lightning averages it weighted by batch size):
+// acc[0] += loss * n_valid, in fp64 (exact: a float times an integer below 2^24), with the loss kernels' clamp of n_valid
+__global__ void loss_accumulate_kernel(const float* __restrict__ loss, const int* __restrict__ n_valid_dev, int B, double* __restrict__ acc) {
+  pdl_trigger();
+  pdl_wait();
+  const int nv = n_valid_dev != nullptr ? min(max(*n_valid_dev, 1), B) : B;
+  acc[0] += (double)loss[0] * (double)nv;
+}
+
+int vitb_train_loss_accumulate(const float* loss, const int* n_valid_dev, int B, double* acc, void* stream) {
+  VITB_REQUIRE(loss && acc, "train_loss_accumulate: null pointer");
+  VITB_REQUIRE(B > 0, "train_loss_accumulate: bad batch size B=%d", B);
+  VITB_LAUNCH((loss_accumulate_kernel), 1, 1, 0, (cudaStream_t)stream, loss, n_valid_dev, B, acc);
+  VITB_LAUNCH_OK();
+  return 0;
+}
+
 int vitb_adam_multi(float* p, const float* g, float* m, float* v, void* w_shadow, int64_t n,
                     const float* hyper_host, const float* hyper_dev, void* stream) {
   VITB_REQUIRE(p && g && m && v, "adam: null pointer");

@@ -35,9 +35,11 @@ from .vit import ViT
 class TrainEngine:
     def __init__(self, model: ViT, batch_size: int, smoothing: float = 0.1, lr: float = 1e-3, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 5e-5, process_group=None, use_graph: bool = True,
-                 overlap_comm: bool = False, mixed_targets: bool = False, optimizer: str = "adam", momentum: Optional[float] = None):
+                 overlap_comm: bool = False, mixed_targets: bool = False, optimizer: str = "adam", momentum: Optional[float] = None,
+                 metrics: bool = False):
         """optimizer: "adam" (network.py:71-77) or "sgd" (network.py:78-84: torch.optim.SGD with momentum = beta1 unless `momentum`
-        is given, coupled weight decay)."""
+        is given, coupled weight decay).  metrics: each step also adds to an epoch record on the device (the correct count of the
+        logits against `labels`, the batch-size-weighted step loss), read by `train_metrics()`; off, the step is unchanged."""
         ops.require_device()
         if optimizer not in ("adam", "sgd"):
             raise NotImplementedError(f"Unknown optimizer: {optimizer}")  # the reference's message (network.py:110)
@@ -149,6 +151,11 @@ class TrainEngine:
         self._n_valid = self.B
         self._next_n_valid = self.B
         self.dlogits = torch.zeros((self.B, model.num_classes), dtype=torch.float32, device=self.dev)
+        # epoch record (metrics=True): [loss_sum, correct, count] of vitb_eval_metrics (its unmixed loss_sum is not reported), then the
+        # sum of step loss * n_valid (vitb_train_loss_accumulate)
+        self.metrics = bool(metrics)
+        self._record = torch.zeros(4, dtype=torch.float64, device=self.dev) if self.metrics else None
+        self._record_ws = torch.zeros(ops.eval_metrics_ws_bytes() // 8, dtype=torch.float64, device=self.dev) if self.metrics else None
         self.logits: Optional[torch.Tensor] = None
         self.hyper_dev = torch.zeros(16, dtype=torch.float32, device=self.dev)
         # nn.Dropout(p) of the blocks (layers.py:35, 38, 102): each block owns a mask stream (seed), the step index is word 10 of
@@ -250,6 +257,9 @@ class TrainEngine:
                       n_valid_dev=n_valid_dev, ws=self._ls_ws)
         else:
             ops.ls_ce(self.logits, self.labels, self.loss, self.dlogits, self.smoothing, 1.0, n_valid_dev=n_valid_dev, ws=self._ls_ws)
+        if self.metrics:  # training accuracy is against the first target (network.py:206)
+            ops.eval_metrics(self.logits, self.labels, self._record[:3], self._record_ws, self.smoothing, n_valid_dev=n_valid_dev)
+            ops.train_loss_accumulate(self.loss, self._record[3:], self.B, n_valid_dev=n_valid_dev)
 
         self._opt_done_from = self.n  # elements [_opt_done_from, n) have had their optimiser step on the side stream
         self._backward(hsaved, saved, words)
@@ -455,6 +465,23 @@ class TrainEngine:
         else:
             self._graph.replay()
         return self.loss
+
+    def train_metrics(self, reset: bool = True) -> Dict[str, float]:
+        """{"loss", "acc", "n"} of the steps since the last reset: the n-weighted mean of the step losses (for CutMix / MixUp batches
+        the mixed objective, network.py:149-167), the accuracy of the logits against the first labels, and the number of images.  One
+        host synchronisation; with a process group the record is first summed over the ranks (a collective: call on all ranks)."""
+        if not self.metrics:
+            raise RuntimeError("construct the engine with metrics=True to keep an epoch record")
+        t = self._record
+        if self.pg is not None and self.world > 1:
+            import torch.distributed as dist
+            t = t.clone()
+            dist.all_reduce(t, group=self.pg)
+        _, correct, n, loss_sum = t.tolist()
+        if reset:
+            self._record.zero_()
+        n = int(n)
+        return {"loss": loss_sum / max(n, 1), "acc": correct / max(n, 1), "n": n}
 
     def sync_weights(self) -> None:
         """Call after writing parameters from outside the step (load_state_dict / load_checkpoint / manual edits on the packed

@@ -249,6 +249,61 @@ def augment_autoaugment(img_u8, dx, dy, flip, code, op_ids, mags, mean, std, out
           "augment_autoaugment")
 
 
+def _check_gather(data_u8, labels_src, idx, out, labels_dst, dx, dy, flip, policy: bool) -> tuple:
+    """Host-side checks of the gather forms: dtype, layout and device of every tensor; returns (N, B, S)."""
+    if data_u8.dtype != torch.uint8 or data_u8.dim() != 4 or data_u8.shape[3] != 3 or data_u8.shape[1] != data_u8.shape[2]:
+        raise ValueError(f"data_u8 must be uint8 (N, S, S, 3) HWC, got {data_u8.dtype} {tuple(data_u8.shape)}")
+    N, S = int(data_u8.shape[0]), int(data_u8.shape[1])
+    if N < 1:
+        raise ValueError("empty dataset: data_u8 has no images")
+    if policy and S > 64:
+        raise ValueError(f"the AutoAugment kernel takes images of at most 64 x 64 pixels, got S={S}")
+    if idx.dtype != torch.int32 or idx.dim() != 1 or idx.numel() < 1:
+        raise ValueError(f"idx must be a non-empty int32 vector, got {idx.dtype} {tuple(idx.shape)}")
+    B = int(idx.numel())
+    if labels_src.dtype != torch.int64 or tuple(labels_src.shape) != (N,):
+        raise ValueError(f"labels_src must be int64 ({N},), got {labels_src.dtype} {tuple(labels_src.shape)}")
+    if out.dtype != torch.float32 or tuple(out.shape) != (B, 3, S, S):
+        raise ValueError(f"out must be float32 ({B}, 3, {S}, {S}), got {out.dtype} {tuple(out.shape)}")
+    if labels_dst.dtype != torch.int64 or tuple(labels_dst.shape) != (B,):
+        raise ValueError(f"labels_dst must be int64 ({B},), got {labels_dst.dtype} {tuple(labels_dst.shape)}")
+    for name, t, dt in (("dx", dx, torch.int32), ("dy", dy, torch.int32), ("flip", flip, torch.uint8)):
+        if t is not None and (t.dtype != dt or tuple(t.shape) != (B,)):
+            raise ValueError(f"{name} must be {dt} ({B},), got {t.dtype} {tuple(t.shape)}")
+    ts = [t for t in (data_u8, labels_src, idx, out, labels_dst, dx, dy, flip) if t is not None]
+    if any(t.device != data_u8.device for t in ts) or not data_u8.is_cuda:
+        raise ValueError("every tensor of a gather must be on the same CUDA device: " + ", ".join(str(t.device) for t in ts))
+    _contig(*ts)
+    return N, B, S
+
+
+def augment_gather(data_u8, labels_src, idx, dx, dy, flip, mean, std, out, labels_dst, pad: int) -> None:
+    """`augment` of the batch data_u8[idx] of a device-resident (N, S, S, 3) dataset, gathered inside the kernel, with
+    labels_dst = labels_src[idx] in the same launch.  A row outside [0, N) gives a NaN image and label -1."""
+    N, B, S = _check_gather(data_u8, labels_src, idx, out, labels_dst, dx, dy, flip, False)
+    m, s_ = _F3(*[float(v) for v in mean]), _F3(*[float(v) for v in std])
+    check(_lib.load().vitb_augment_crop_flip_normalize_gather(_ptr(data_u8), _ptr(labels_src), N, _ptr(idx), _ptr(dx), _ptr(dy), _ptr(flip),
+                                                              C.cast(m, C.c_void_p), C.cast(s_, C.c_void_p), _ptr(out), _ptr(labels_dst), B, S,
+                                                              int(pad), _stream()), "augment_crop_flip_normalize_gather")
+
+
+def augment_autoaugment_gather(data_u8, labels_src, idx, dx, dy, flip, code, op_ids, mags, mean, std, out, labels_dst, pad: int) -> None:
+    """`augment_autoaugment` of the batch data_u8[idx], gathered inside the kernel, as `augment_gather`."""
+    N, B, S = _check_gather(data_u8, labels_src, idx, out, labels_dst, dx, dy, flip, True)
+    if code.dtype != torch.int32 or tuple(code.shape) != (B,) or code.device != data_u8.device:
+        raise ValueError(f"code must be int32 ({B},) on {data_u8.device}, got {code.dtype} {tuple(code.shape)} on {code.device}")
+    if len(op_ids) != len(mags) or len(op_ids) % 2 != 0:
+        raise ValueError("op_ids and mags: two entries per sub-policy")
+    _contig(code)
+    m, s_ = _F3(*[float(v) for v in mean]), _F3(*[float(v) for v in std])
+    n = len(op_ids)
+    ids, mg = (C.c_int32 * n)(*[int(v) for v in op_ids]), (C.c_double * n)(*[float(v) for v in mags])
+    check(_lib.load().vitb_augment_autoaugment_gather(_ptr(data_u8), _ptr(labels_src), N, _ptr(idx), _ptr(dx), _ptr(dy), _ptr(flip), _ptr(code),
+                                                      C.cast(ids, C.c_void_p), C.cast(mg, C.c_void_p), n // 2, C.cast(m, C.c_void_p),
+                                                      C.cast(s_, C.c_void_p), _ptr(out), _ptr(labels_dst), B, S, int(pad), _stream()),
+          "augment_autoaugment_gather")
+
+
 def batch_mix(img, perm, out, mode: int, lam: float = 1.0, box=(0, 0, 0, 0)) -> None:
     """CutMix (mode 0: paste rows box[0]:box[1], columns box[2]:box[3] of img[perm[b]] into img[b], da.py:68) or MixUp (mode 1:
     lam * img + (1 - lam) * img[perm], da.py:90) of an fp32 (B, C, S, S) batch into `out`."""
@@ -432,3 +487,10 @@ def dp_reduce_adam(g: PeerPointers, p: PeerPointers, shadow: Optional[PeerPointe
                                           int(n), int(rank), int(world), int(optimizer), C.cast(hh, C.c_void_p) if hh is not None else None,
                                           _ptr(hyper_dev), _stream()),
           "dp_reduce_adam")
+
+
+def train_loss_accumulate(loss, acc, B: int, n_valid_dev=None) -> None:
+    """acc[0] += loss * n_valid in fp64 (`loss`: the 1-float device result of `ls_ce`; n_valid clamped to [1, B] as there)."""
+    assert loss.dtype == torch.float32 and loss.numel() == 1 and acc.dtype == torch.float64 and acc.numel() >= 1
+    assert n_valid_dev is None or n_valid_dev.dtype == torch.int32
+    check(_lib.load().vitb_train_loss_accumulate(_ptr(loss), _ptr(n_valid_dev), int(B), _ptr(acc), _stream()), "train_loss_accumulate")

@@ -132,18 +132,41 @@ class GpuAugment:
         code = sub | (g[:, 0] << 8) | (g[:, 1] << 9) | (s[:, 0] << 10) | (s[:, 1] << 11)
         return dx, dy, fl, code
 
-    def __call__(self, img_u8: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def __call__(self, img_u8: torch.Tensor, out: Optional[torch.Tensor] = None, index: Optional[torch.Tensor] = None,
+                 labels: Optional[torch.Tensor] = None, labels_out: Optional[torch.Tensor] = None):
+        """Transform the uint8 (B, S, S, 3) batch `img_u8` into fp32 (B, 3, S, S) `out` (allocated when None) and return it.
+
+        With `index` (int32 (B,) on the device), `img_u8` is a resident (N, S, S, 3) dataset and `labels` its int64 (N,) labels:
+        the batch is rows index[0..B) of it, gathered inside the same kernel, with the same draws as for the contiguous batch
+        img_u8[index].  Returns (out, labels_out), labels_out[i] = labels[index[i]] (allocated when None).  A row outside [0, N)
+        comes out as a NaN image with label -1."""
         from . import ops
-        B = img_u8.shape[0]
+        if index is None:
+            B = img_u8.shape[0]
+            if out is None:
+                out = torch.empty((B, 3, self.size, self.size), dtype=torch.float32, device=img_u8.device)
+            if self.policy is None:
+                dx, dy, fl = self.draw(B, img_u8.device)
+                ops.augment(img_u8, dx, dy, fl, self.mean, self.std, out, self.padding)
+            else:
+                dx, dy, fl, code = self.draw(B, img_u8.device)
+                ops.augment_autoaugment(img_u8, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, self.padding)
+            return out
+        if labels is None:
+            raise ValueError("index= gathers from a dataset: give its labels= too")
+        B, dev = int(index.numel()), img_u8.device
         if out is None:
-            out = torch.empty((B, 3, self.size, self.size), dtype=torch.float32, device=img_u8.device)
+            out = torch.empty((B, 3, self.size, self.size), dtype=torch.float32, device=dev)
+        if labels_out is None:
+            labels_out = torch.empty((B,), dtype=torch.int64, device=dev)
         if self.policy is None:
-            dx, dy, fl = self.draw(B, img_u8.device)
-            ops.augment(img_u8, dx, dy, fl, self.mean, self.std, out, self.padding)
+            dx, dy, fl = self.draw(B, dev)
+            ops.augment_gather(img_u8, labels, index, dx, dy, fl, self.mean, self.std, out, labels_out, self.padding)
         else:
-            dx, dy, fl, code = self.draw(B, img_u8.device)
-            ops.augment_autoaugment(img_u8, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, self.padding)
-        return out
+            dx, dy, fl, code = self.draw(B, dev)
+            ops.augment_autoaugment_gather(img_u8, labels, index, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, labels_out,
+                                           self.padding)
+        return out, labels_out
 
 
 # ---------------------------------------------------------------------------------------------

@@ -10,6 +10,8 @@ Public surface (mirrors the reference's module/class names for this path):
   TrainEngine                                           (the per-batch hot loop, CUDA-graphed, data-parallel)
   EvalEngine                                            (the validation pass, network.py:388-395: forward-only CUDA graph,
                                                          loss / accuracy summed on the device, one host sync per pass)
+  DeviceDataset, DeviceLoader                           (the DataLoader / DistributedSampler of utils.py:452-470 over a
+                                                         dataset resident in device memory)
   set_precision / get_precision                         ('bf16' tensor-core path or 'fp32' check mode)
   WarmupCosine, evaluate, save_checkpoint, load_checkpoint   (network.py:113-122, 388-395; main.py:234-237, run_model.py:12-37)
 """
@@ -24,5 +26,6 @@ from .criterions import LabelSmoothingCrossEntropyLoss  # noqa: E402,F401
 from .optim import FusedAdam, adam_hyper, sgd_hyper  # noqa: E402,F401
 from .engine import TrainEngine  # noqa: E402,F401
 from .evaluator import EvalEngine  # noqa: E402,F401
+from .loader import DeviceDataset, DeviceLoader  # noqa: E402,F401
 from .schedule import (WarmupCosine, warmup_cosine_lr, evaluate, save_checkpoint, load_checkpoint, to_lightning_checkpoint,  # noqa: E402,F401
                        GpuAugment, GpuCutMix, GpuMixUp, cutmix_box)
