@@ -165,6 +165,16 @@ int vitb_augment_autoaugment_gather(const uint8_t* data_u8, const int64_t* label
                                     const int32_t* op_ids, const double* mags, int n_sub, const float* mean3, const float* std3,
                                     float* out, int64_t* labels_dst, int B, int S, int pad, void* stream);
 
+/* ---- RandomCropPaste: the reference's da.RandomCropPaste(size) (alpha = 1, flip_p = 0.5), which utils.get_transform appends after
+ * ToTensor + Normalize with --rcpaste; it replaces, per image,
+ *     front = img[:, fy1:fy1+fh, fx1:fx1+fw].clone(); [front = front.flip(-1)]; [img = img.flip(-1)]
+ *     img[:, y1:y1+fh, x1:x1+fw] *= a;  img[:, y1:y1+fh, x1:x1+fw] += front * (1 - a)
+ * In place on img fp32 (B,3,S,S) device.  params int32 (B,8) device: [fx1, fy1, fw, fh, x1, y1, flip_front, flip_img] per image;
+ * alpha double (B) device: a.  The caller draws and derives them.  As in the reference, whose a is a float64 array, the blend is fp64:
+ * out = (float)((double)(float)(base * a) + front * (1 - a)).  fw = 0 or fh = 0: only the whole-image flip.  A box that does not lie
+ * inside the image makes that image NaN.  1 <= S <= 64 (the image is staged in 3*S*S floats of shared memory). ---- */
+int vitb_random_crop_paste(float* img, const int32_t* params, const double* alpha, int B, int S, void* stream);
+
 /* ---- batch-level CutMix / MixUp (da.py:51-93; network.py:149-158) on a normalised fp32 (B, C, S, S) device batch; perm int32 (B) =
  * the shuffled partner of every image (the caller draws it, with lam and the box, like the reference does on the host).
  * mode 0: out[b, :, i, j] = img[perm[b], :, i, j] inside rows x1 <= i < x2, columns y1 <= j < y2 (the reference's own index order,

@@ -1,12 +1,14 @@
-"""Train the ViT on CIFAR-10 / CIFAR-100 with the reference's recipe (main.py + network.py), every step on the device.
+"""Train the ViT on CIFAR-10 / CIFAR-100 / SVHN with the reference's recipe (main.py + network.py), every step on the device.
 
-    python tools/train.py --data-root DIR [--dataset c10|c100] [--autoaugment] [--label-smoothing] [--cutmix | --mixup] ...
+    python tools/train.py --data-root DIR [--dataset c10|c100|svhn] [--autoaugment] [--rcpaste] [--label-smoothing] [--cutmix | --mixup] ...
     python tools/train.py --synthetic 5000 --max-epochs 2 ...            (a seeded, learnable uint8 set: tests, benchmarks)
     torchrun --nproc-per-node 8 tools/train.py ...                        (one process per GPU)
 
 Data: the python-pickle batches from --data-root (cifar-10-batches-py/data_batch_1..5 + test_batch; cifar-100-python/train + test,
-fine labels).  Nothing is downloaded.  Both sets are uploaded once (DeviceDataset); an epoch is one DeviceLoader pass (the
-DistributedSampler order, batches gathered inside the augmentation kernel) through TrainEngine(metrics=True), then EvalEngine on
+fine labels), or SVHN's train_32x32.mat + test_32x32.mat where torchvision.datasets.SVHN keeps them (no `extra` split).  Nothing is
+downloaded.  The augmentation is get_transform's for the dataset: RandomCrop(32, 4), the flip (not for SVHN), with --autoaugment the
+dataset's policy (CIFAR10Policy for both CIFARs, SVHNPolicy), Normalize with the dataset's mean / std, with --rcpaste RandomCropPaste.
+Both sets are uploaded once (DeviceDataset); an epoch is one DeviceLoader pass (the DistributedSampler order, batches gathered inside the augmentation kernel) through TrainEngine(metrics=True), then EvalEngine on
 the resident test set.  Per epoch, as network.py does: the warm-up + cosine learning rate (network.py:113-122), the NaN check of
 the parameters (network.py:226-228), the best-val_loss checkpoint (ModelCheckpoint(monitor="val_loss", save_top_k=1),
 main.py:213-219) and one JSON line on stdout.  At the end the reference's checkpoint (main.py:234-237).  Flag names and defaults
@@ -27,7 +29,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-NUM_CLASSES = {"c10": 10, "c100": 100}
+NUM_CLASSES = {"c10": 10, "c100": 100, "svhn": 10}
 
 
 def parse_args(argv=None):
@@ -48,6 +50,7 @@ def parse_args(argv=None):
     ap.add_argument("--label-smoothing", action="store_true")
     ap.add_argument("--smoothing", type=float, default=0.1)
     ap.add_argument("--autoaugment", action="store_true")
+    ap.add_argument("--rcpaste", action="store_true")
     ap.add_argument("--cutmix", action="store_true")
     ap.add_argument("--mixup", action="store_true")
     ap.add_argument("--dropout", type=float, default=0.0)
@@ -103,6 +106,32 @@ def read_cifar(root: str, dataset: str):
     return tuple(out)
 
 
+def read_svhn(root: str):
+    """((train_images, train_labels), (test_images, test_labels)) from train_32x32.mat / test_32x32.mat under `root`, as
+    torchvision.datasets.SVHN reads them: X (32, 32, 3, N) becomes uint8 (N, 32, 32, 3) HWC, labels int64 with 10 -> 0.  Raises
+    FileNotFoundError naming what is missing."""
+    from scipy.io import loadmat
+    files = [os.path.join(root, f"{split}_32x32.mat") for split in ("train", "test")]
+    missing = [f for f in files if not os.path.isfile(f)]
+    if missing:
+        raise FileNotFoundError(f"SVHN .mat files not found (this tool downloads nothing): {', '.join(missing)}")
+    out = []
+    for f in files:
+        m = loadmat(f)
+        y = m["y"].astype(np.int64).squeeze(1)
+        y[y == 10] = 0
+        out.append((np.ascontiguousarray(np.asarray(m["X"], dtype=np.uint8).transpose(3, 0, 1, 2)), y))
+    return tuple(out)
+
+
+def augment_recipe(dataset: str, autoaugment: bool) -> dict:
+    """GpuAugment's keyword arguments for get_transform's training pipeline of `dataset` (without the seed and --rcpaste)."""
+    from vit_cifar_b200.schedule import CIFAR10_MEAN, CIFAR10_STD, CIFAR100_MEAN, CIFAR100_STD, SVHN_MEAN, SVHN_STD
+    mean, std = {"c10": (CIFAR10_MEAN, CIFAR10_STD), "c100": (CIFAR100_MEAN, CIFAR100_STD), "svhn": (SVHN_MEAN, SVHN_STD)}[dataset]
+    policy = ("svhn" if dataset == "svhn" else "cifar10") if autoaugment else None
+    return dict(mean=mean, std=std, flip=dataset != "svhn", policy=policy)
+
+
 def synthetic_set(n: int, num_classes: int, seed: int, size: int = 32):
     """A seeded uint8 (n, size, size, 3) set a ViT can learn: each class is a fixed random colour pattern plus noise."""
     rng = np.random.default_rng(seed)
@@ -129,7 +158,6 @@ def main(argv=None):
     args = parse_args(argv)
     import torch
     import vit_cifar_b200 as vb
-    from vit_cifar_b200.schedule import CIFAR10_MEAN, CIFAR10_STD, CIFAR100_MEAN, CIFAR100_STD
 
     pg, rank, world = None, 0, 1
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -140,14 +168,15 @@ def main(argv=None):
         pg, rank, world = dist.group.WORLD, dist.get_rank(), dist.get_world_size()
     torch.manual_seed(args.seed)
     np.random.seed(args.seed)
-    mean, std = (CIFAR10_MEAN, CIFAR10_STD) if args.dataset == "c10" else (CIFAR100_MEAN, CIFAR100_STD)
+    recipe = augment_recipe(args.dataset, args.autoaugment)
+    mean, std = recipe["mean"], recipe["std"]
 
     if args.synthetic:
         train = synthetic_set(args.synthetic, args.num_classes, args.seed)
         test = synthetic_set(max(args.synthetic // 5, 1), args.num_classes, args.seed + 1)
     else:
         try:
-            train, test = read_cifar(args.data_root, args.dataset)
+            train, test = read_svhn(args.data_root) if args.dataset == "svhn" else read_cifar(args.data_root, args.dataset)
         except FileNotFoundError as e:
             print(f"error: {e}", file=sys.stderr)
             return 2
@@ -161,7 +190,7 @@ def main(argv=None):
     engine = vb.TrainEngine(model, args.batch_size, smoothing=smoothing, lr=args.lr, betas=(args.beta1, args.beta2),
                             weight_decay=args.weight_decay, process_group=pg, mixed_targets=mixed, optimizer=args.optimizer, metrics=True)
     evaluator = vb.EvalEngine(model, batch_size=args.eval_batch_size, smoothing=smoothing, mean=mean, std=std, process_group=pg)
-    aug = vb.GpuAugment(S, 4, mean, std, seed=args.seed + rank, policy="cifar10" if args.autoaugment else None)
+    aug = vb.GpuAugment(S, 4, seed=args.seed + rank, rcpaste=args.rcpaste, **recipe)
     mix = vb.GpuCutMix(S, beta=1.0) if args.cutmix else MaybeMixUp(vb.GpuMixUp(alpha=1.0)) if args.mixup else None
     loader = vb.DeviceLoader(train_ds, args.batch_size, shuffle=True, seed=args.seed, augment=aug, mix=mix, process_group=pg)
     val_loader = vb.DeviceLoader(test_ds, args.eval_batch_size, shuffle=False, process_group=pg)

@@ -63,6 +63,7 @@ SIGNATURES = {
     "vitb_augment_autoaugment": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i, _i, _i, _p]),
     "vitb_augment_crop_flip_normalize_gather": (_i, [_p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p]),
     "vitb_augment_autoaugment_gather": (_i, [_p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _p]),
+    "vitb_random_crop_paste": (_i, [_p, _p, _p, _i, _i, _p]),
     "vitb_batch_mix": (_i, [_p, _p, _p, _i, _i, _i, _i, C.c_double, _i, _i, _i, _i, _p]),
     "vitb_dropout_threshold": (C.c_uint32, [_f]),
     "vitb_dropout": (_i, [_p, _p, _p, _i64, _f, C.c_uint64, C.c_uint32, C.c_uint32, _p, _i, _p]),

@@ -291,6 +291,47 @@ __global__ void __launch_bounds__(kAaThreads)
       o[(int64_t)c * NP + p] = bad ? __int_as_float(0x7fffffff) : __fdiv_rn(__fsub_rn(__fmul_rn((float)cur[p * 3 + c], 1.0f / 255.0f), mc[c]), sc[c]);
 }
 
+// RandomCropPaste (the reference's da.RandomCropPaste, the last transform of get_transform with --rcpaste), in place on normalised
+// fp32 (B, 3, S, S).  One CTA per image stages the whole image in shared memory (3 S^2 floats: 48 KB at S = kCpMaxS), because every
+// output pixel reads two input pixels: the (flipped) base and, inside the paste box, the front pixel taken before the whole-image flip.
+// params[b] = [fx1, fy1, fw, fh, x1, y1, flip_front, flip_img]; a[b] = the blend weight.  The reference blends with a float64 array,
+// so torch computes in fp64: out = fp32(fp64(fp32(base * a)) + front * (1 - a)), written with _rn intrinsics so that nothing is
+// contracted into an FMA.  Parameters that would read or write outside the image give a NaN image (no synchronous error exists).
+constexpr int kCpMaxS = 64;
+constexpr int kCpThreads = 256;
+
+__global__ void __launch_bounds__(kCpThreads)
+    random_crop_paste_kernel(float* __restrict__ img, const int32_t* __restrict__ params, const double* __restrict__ alpha, int S) {
+  extern __shared__ float stage[];
+  const int NP = S * S, b = blockIdx.x, tid = threadIdx.x;
+  float* im = img + (int64_t)b * 3 * NP;
+  pdl_trigger();
+  pdl_wait();
+  const int32_t* pr = params + b * 8;
+  const int fx1 = pr[0], fy1 = pr[1], fw = pr[2], fh = pr[3], x1 = pr[4], y1 = pr[5];
+  const bool flip_front = pr[6] != 0, flip_img = pr[7] != 0;
+  const double a = alpha[b], na = __dsub_rn(1.0, a);
+  const bool bad = fw < 0 || fh < 0 || fx1 < 0 || fy1 < 0 || x1 < 0 || y1 < 0 || fx1 > S - fw || fy1 > S - fh || x1 > S - fw || y1 > S - fh;
+  if (bad) {
+    for (int i = tid; i < 3 * NP; i += blockDim.x) im[i] = __int_as_float(0x7fffffff);
+    return;
+  }
+  for (int i = tid; i < 3 * NP; i += blockDim.x) stage[i] = im[i];
+  __syncthreads();
+  for (int i = tid; i < 3 * NP; i += blockDim.x) {
+    const int c = i / NP, y = (i % NP) / S, x = i % S;
+    const float* ch = stage + c * NP;
+    float v = ch[y * S + (flip_img ? S - 1 - x : x)];
+    if (x >= x1 && x < x1 + fw && y >= y1 && y < y1 + fh) {
+      const int u = flip_front ? fw - 1 - (x - x1) : x - x1;
+      const float f = ch[(fy1 + y - y1) * S + fx1 + u];
+      const double scaled = (double)__double2float_rn(__dmul_rn((double)v, a));
+      v = __double2float_rn(__dadd_rn(scaled, __dmul_rn((double)f, na)));
+    }
+    im[i] = v;
+  }
+}
+
 // Python's round(x, 15): the double nearest to x rounded to 15 decimals (both directions correctly rounded)
 double round15(double x) {
   char buf[64];
@@ -367,4 +408,12 @@ int vitb_augment_autoaugment_gather(const uint8_t* data_u8, const int64_t* label
                "augment_autoaugment_gather: null pointer");
   VITB_REQUIRE(N > 0, "augment_autoaugment_gather: empty dataset (N=%d)", N);
   return launch_autoaugment(data_u8, idx, N, labels_src, labels_dst, dx, dy, flip, code, op_ids, mags, n_sub, mean3, std3, out, B, S, pad, stream);
+}
+
+int vitb_random_crop_paste(float* img, const int32_t* params, const double* alpha, int B, int S, void* stream) {
+  VITB_REQUIRE(img && params && alpha, "random_crop_paste: null pointer");
+  VITB_REQUIRE(B > 0 && S > 0 && S <= kCpMaxS, "random_crop_paste: bad shape B=%d S=%d (S <= %d)", B, S, kCpMaxS);
+  VITB_LAUNCH((random_crop_paste_kernel), B, kCpThreads, (size_t)3 * S * S * sizeof(float), (cudaStream_t)stream, img, params, alpha, S);
+  VITB_LAUNCH_OK();
+  return 0;
 }

@@ -304,6 +304,27 @@ def augment_autoaugment_gather(data_u8, labels_src, idx, dx, dy, flip, code, op_
           "augment_autoaugment_gather")
 
 
+CROP_PASTE_MAX_S = 64  # vitb_random_crop_paste stages an image in 3 * S * S floats of shared memory
+
+
+def random_crop_paste(img, params, alpha) -> None:
+    """da.RandomCropPaste in place on a normalised fp32 (B, 3, S, S) device batch, for given draws: params int32 (B, 8) =
+    [fx1, fy1, fw, fh, x1, y1, flip_front, flip_img] per image, alpha float64 (B,) = the blend weight a (vitb_random_crop_paste)."""
+    if img.dtype != torch.float32 or img.dim() != 4 or img.shape[1] != 3 or img.shape[2] != img.shape[3] or img.shape[0] < 1:
+        raise ValueError(f"img must be a non-empty float32 (B, 3, S, S) batch, got {img.dtype} {tuple(img.shape)}")
+    B, S = int(img.shape[0]), int(img.shape[2])
+    if S > CROP_PASTE_MAX_S:
+        raise ValueError(f"the crop-paste kernel takes images of at most {CROP_PASTE_MAX_S} x {CROP_PASTE_MAX_S} pixels, got S={S}")
+    if params.dtype != torch.int32 or tuple(params.shape) != (B, 8):
+        raise ValueError(f"params must be int32 ({B}, 8), got {params.dtype} {tuple(params.shape)}")
+    if alpha.dtype != torch.float64 or tuple(alpha.shape) != (B,):
+        raise ValueError(f"alpha must be float64 ({B},), got {alpha.dtype} {tuple(alpha.shape)}")
+    if not img.is_cuda or params.device != img.device or alpha.device != img.device:
+        raise ValueError(f"img, params and alpha must be on the same CUDA device: {img.device}, {params.device}, {alpha.device}")
+    _contig(img, params, alpha)
+    check(_lib.load().vitb_random_crop_paste(_ptr(img), _ptr(params), _ptr(alpha), B, S, _stream()), "random_crop_paste")
+
+
 def batch_mix(img, perm, out, mode: int, lam: float = 1.0, box=(0, 0, 0, 0)) -> None:
     """CutMix (mode 0: paste rows box[0]:box[1], columns box[2]:box[3] of img[perm[b]] into img[b], da.py:68) or MixUp (mode 1:
     lam * img + (1 - lam) * img[perm], da.py:90) of an fp32 (B, C, S, S) batch into `out`."""

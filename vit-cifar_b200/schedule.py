@@ -87,11 +87,28 @@ def load_checkpoint(model, ckpt, strict: bool = False, prefix: str = "model."):
 # ---------------------------------------------------------------------------------------------
 CIFAR10_MEAN, CIFAR10_STD = (0.4914, 0.4822, 0.4465), (0.2470, 0.2435, 0.2616)      # utils.py:380
 CIFAR100_MEAN, CIFAR100_STD = (0.5071, 0.4867, 0.4408), (0.2675, 0.2565, 0.2761)    # utils.py:470
+# utils.py, the svhn branch of get_dataloader: as remembered from the reference, not yet compared with its source
+SVHN_MEAN, SVHN_STD = (0.4377, 0.4438, 0.4728), (0.1980, 0.2010, 0.1970)
+
+
+def crop_paste_box(S: int, lam: torch.Tensor, cx: torch.Tensor, cy: torch.Tensor, ux: torch.Tensor, uy: torch.Tensor) -> torch.Tensor:
+    """da.RandomCropPaste's box arithmetic for B images as int32 (B, 6) [fx1, fy1, fw, fh, x1, y1]: lam (float64) ~ Beta(1, 1),
+    cx / cy the box centres (integers in [0, S)), ux / uy float64 uniforms in [0, 1) for the paste corner.
+        cut = np.int(S * np.sqrt(1 - lam)); f?1, f?2 = clip(c? - cut // 2, 0, S), clip(c? + cut // 2, 0, S)   (_rand_bbox)
+        x1 = randint(0, S - fw) = floor(ux * (S - fw)), y1 likewise
+    fw == S (lam == 0 exactly) makes the reference's randint(0, 0) raise; here the paste starts at 0."""
+    cut = torch.floor(S * torch.sqrt(1.0 - lam)).to(torch.int64)
+    c = torch.stack((cx, cy), 1).to(torch.int64)
+    half = (cut // 2)[:, None]
+    lo, hi = (c - half).clamp(0, S), (c + half).clamp(0, S)
+    w = hi - lo
+    corner = torch.floor(torch.stack((ux, uy), 1) * (S - w)).to(torch.int64)
+    return torch.cat((lo, w, corner), 1).to(torch.int32)
 
 
 class GpuAugment:
     """get_transform's training pipeline — RandomCrop(size, padding) + RandomHorizontalFlip + [AutoAugment policy] + ToTensor +
-    Normalize(mean, std) — on a raw uint8 (B, S, S, 3) batch that is already on the device: one kernel instead of a per-image PIL
+    Normalize(mean, std) [+ RandomCropPaste] — on a raw uint8 (B, S, S, 3) batch that is already on the device: one kernel instead of a per-image PIL
     pipeline in DataLoader workers, and 4x fewer bytes over PCIe than normalised fp32 batches.
     The random draws use a torch.Generator on the device (torchvision and the reference draw them on the host, per image).
 
@@ -101,14 +118,22 @@ class GpuAugment:
         svhn         GpuAugment(32, 4, mean, std, flip=False, policy="svhn")
     With a policy, each image also draws its sub-policy (uniform), the two gates (rand < p) and two signs (+-1, p = 1/2) after the
     crop and flip draws; every op reproduces the Pillow call of the reference's autoaugment.py (csrc/augment.cu).  The draws follow
-    the reference's distribution, not Python's `random` stream."""
+    the reference's distribution, not Python's `random` stream.
+
+    rcpaste=True (main.py --rcpaste) appends da.RandomCropPaste(size): a second kernel pass over `out`, in place
+    (csrc/augment.cu), with its draws (draw_crop_paste) taken after all the others of the batch.  size <= 64."""
 
     def __init__(self, size: int = 32, padding: int = 4, mean=CIFAR10_MEAN, std=CIFAR10_STD, flip: bool = True, seed: int = 0,
-                 device="cuda", policy: Optional[str] = None):
+                 device="cuda", policy: Optional[str] = None, rcpaste: bool = False):
         self.size, self.padding, self.mean, self.std, self.flip = int(size), int(padding), tuple(mean), tuple(std), bool(flip)
         self.gen = torch.Generator(device=device)
         self.gen.manual_seed(seed)
         self.policy = policy
+        self.rcpaste = bool(rcpaste)
+        if self.rcpaste:
+            from .ops import CROP_PASTE_MAX_S
+            if self.size > CROP_PASTE_MAX_S:
+                raise ValueError(f"rcpaste=True takes images of at most {CROP_PASTE_MAX_S} x {CROP_PASTE_MAX_S} pixels, got size={self.size}")
         if policy is not None:
             from .autoaugment import POLICIES, kernel_table
             if policy not in POLICIES:
@@ -132,6 +157,17 @@ class GpuAugment:
         code = sub | (g[:, 0] << 8) | (g[:, 1] << 9) | (s[:, 0] << 10) | (s[:, 1] << 11)
         return dx, dy, fl, code
 
+    def draw_crop_paste(self, B: int, device):
+        """(params, a) of da.RandomCropPaste(size) for B images, as vitb_random_crop_paste reads them: params int32 (B, 8) =
+        [fx1, fy1, fw, fh, x1, y1, flip_front, flip_img], a float64 (B,).  lam ~ Beta(1, 1) = U[0, 1), the box centres uniform
+        over [0, S), the paste corner uniform over [0, S - fw) x [0, S - fh), each flip rand <= 0.5 and a ~ U[0, 1), as the
+        reference draws them (not numpy's stream).  On the device, without a host synchronisation."""
+        u = torch.rand((B, 6), generator=self.gen, device=device, dtype=torch.float64)  # lam, ux, uy, two flips, a
+        c = torch.randint(0, self.size, (B, 2), generator=self.gen, device=device)
+        box = crop_paste_box(self.size, u[:, 0], c[:, 0], c[:, 1], u[:, 1], u[:, 2])
+        params = torch.cat((box, (u[:, 3:5] <= 0.5).to(torch.int32)), 1)
+        return params, u[:, 5].contiguous()
+
     def __call__(self, img_u8: torch.Tensor, out: Optional[torch.Tensor] = None, index: Optional[torch.Tensor] = None,
                  labels: Optional[torch.Tensor] = None, labels_out: Optional[torch.Tensor] = None):
         """Transform the uint8 (B, S, S, 3) batch `img_u8` into fp32 (B, 3, S, S) `out` (allocated when None) and return it.
@@ -151,6 +187,8 @@ class GpuAugment:
             else:
                 dx, dy, fl, code = self.draw(B, img_u8.device)
                 ops.augment_autoaugment(img_u8, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, self.padding)
+            if self.rcpaste:
+                ops.random_crop_paste(out, *self.draw_crop_paste(B, img_u8.device))
             return out
         if labels is None:
             raise ValueError("index= gathers from a dataset: give its labels= too")
@@ -166,6 +204,8 @@ class GpuAugment:
             dx, dy, fl, code = self.draw(B, dev)
             ops.augment_autoaugment_gather(img_u8, labels, index, dx, dy, fl, code, self.op_ids, self.mags, self.mean, self.std, out, labels_out,
                                            self.padding)
+        if self.rcpaste:
+            ops.random_crop_paste(out, *self.draw_crop_paste(B, dev))
         return out, labels_out
 
 
@@ -201,7 +241,7 @@ class GpuCutMix:
         r_x = np.random.uniform(0, self.size)
         r_y = np.random.uniform(0, self.size)
         box, lambda_ = cutmix_box(self.size, lambda_, r_x, r_y)
-        idx = rand_idx.to(img.device)
+        idx = rand_idx.pin_memory().to(img.device, non_blocking=True)  # from pageable memory the copy would wait for the device
         out = torch.empty_like(img)
         ops.batch_mix(img, idx.to(torch.int32), out, 0, 1.0, box)
         return out, label, label[idx], lambda_
