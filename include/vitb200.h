@@ -75,7 +75,8 @@ int vitb_patch_embed_bwd(const float* img, const void* words, const void* dout, 
 
 /* ---- LayerNorm: layers.py:26,30,45,47 (la1/la2), vit.py:62 (fc[0]); eps 1e-5, affine ----
  * x act, row r at x + r*x_row_stride elements (lets the head read out[:,0], vit.py:73); y act (rows,H)
- * mean/rstd fp32 (rows) saved for backward. */
+ * mean/rstd fp32 (rows) saved for backward.  H: a multiple of 64 up to 1024 (H % 128 == 64 runs two-element lane
+ * groups); the row strides a multiple of 4.  The backward entry points take the same widths. */
 int vitb_layernorm_fwd(const void* x, int64_t x_row_stride, const float* gamma, const float* beta,
                        void* y, float* mean, float* rstd, int rows, int H, float eps, int dt,
                        void* stream);
@@ -93,7 +94,9 @@ int vitb_layernorm_bwd(const void* dy, const void* x, int64_t x_row_stride, cons
  *      vit.py:63,76 (fc[1]).  GELU is exact/erf (nn.GELU default).
  * C[M,N] = act(A[M,K] · W[N,K]ᵀ + bias[N]) (+ residual[M,N]);  if preact != NULL the value before
  * GELU is stored there (needed by backward).  flags: VITB_GEMM_GELU.  A,W,residual,C,preact: act type.
- * bf16: tcgen05 path, needs N % 128 == 0 and K % 64 == 0 (else falls to the SIMT kernel). */
+ * bf16: tcgen05 path when M >= 32, N % 64 == 0 and K % 8 == 0 (N % 128 == 64: a partial last 128-column tile); other
+ * shapes and fp32 run the SIMT kernel.  The same holds for the output width K of vitb_gemm_dgrad, and vitb_gemm_wgrad_dbias
+ * takes N and K multiples of 64 on the tensor cores. */
 #define VITB_GEMM_GELU 1
 #define VITB_GEMM_OUT_F32 2 /* C is fp32 regardless of dt (head logits) */
 int vitb_gemm_bias_act_fwd(const void* a, const void* w_act, const float* bias, const void* residual,

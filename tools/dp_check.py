@@ -52,7 +52,9 @@ def main():
     ok = True
     tiny = dict(num_classes=10, patch=8, num_layers=2, hidden=128, mlp_hidden=128, head=4)
     cases = [("tiny fp32", tiny, 8, "fp32", False, "adam"), ("tiny fp32 sgd graph", tiny, 8, "fp32", True, "sgd"),
-             ("bench bf16 graph", dict(num_classes=10, patch=8, num_layers=7, hidden=384, mlp_hidden=384, head=12), 1024, "bf16", True, "adam")]
+             ("bench bf16 graph", dict(num_classes=10, patch=8, num_layers=7, hidden=384, mlp_hidden=384, head=12), 1024, "bf16", True, "adam"),
+             ("vit-tiny width 192 bf16 graph", dict(num_classes=10, patch=8, num_layers=2, hidden=192, mlp_hidden=768, head=3), 256, "bf16", True,
+              "adam")]
     for name, cfg, B, precision, graph, optimizer in cases:
         p_ref, l_ref, ms_ref = run(cfg, B, "single", 4, graph, precision, optimizer)
         p_fus, l_fus, ms_fus = run(cfg, B, "fused", 4, graph, precision, optimizer)

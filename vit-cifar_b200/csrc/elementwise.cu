@@ -347,6 +347,196 @@ static int ln_bwd_blocks(int rows) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// LayerNorm at H = 64 * VEC with VEC odd (H % 128 == 64: 64, 192, 320, ..., 960): the same one-warp-per-row kernels with
+// two-element lane groups, VEC pairs per lane at columns (i * 32 + lane) * 2.  The four-element kernels above serve every
+// H % 128 == 0 and are not touched by these.
+// ---------------------------------------------------------------------------------------------
+template <typename T> struct Raw2;
+template <> struct Raw2<float> { float2 v; };
+template <> struct Raw2<bf16> { uint32_t v; };
+__device__ __forceinline__ Raw2<float> ldraw2(const float* p) { Raw2<float> r; r.v = *reinterpret_cast<const float2*>(p); return r; }
+__device__ __forceinline__ Raw2<bf16> ldraw2(const bf16* p) { Raw2<bf16> r; r.v = *reinterpret_cast<const uint32_t*>(p); return r; }
+__device__ __forceinline__ float2 cvt2(const Raw2<float>& r) { return r.v; }
+__device__ __forceinline__ float2 cvt2(const Raw2<bf16>& r) { return unpack_bf16x2(r.v); }
+__device__ __forceinline__ float2 ld2f(const float* p) { return *reinterpret_cast<const float2*>(p); }
+__device__ __forceinline__ void st2(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+__device__ __forceinline__ void st2(bf16* p, float2 v) { *reinterpret_cast<uint32_t*>(p) = pack_bf16x2(v.x, v.y); }
+// two consecutive elements starting at flat element index e (a multiple of 2): a quarter of a mask group
+__device__ __forceinline__ void drop_apply2(float2& v, const DropParams& d, uint32_t step, uint64_t e) {
+  const uint4 r = drop_words(d, step, e >> 3);
+  const uint32_t q = (uint32_t)(e >> 1) & 3u;
+  const uint32_t w = q == 0 ? r.x : (q == 1 ? r.y : (q == 2 ? r.z : r.w));
+  v.x = drop_one(v.x, w, 0, d.thr, d.scale);
+  v.y = drop_one(v.y, w, 1, d.thr, d.scale);
+}
+
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256, 4) ln_fwd_pair_kernel(const T* __restrict__ x, int64_t xs, const float* __restrict__ gamma,
+                                                          const float* __restrict__ beta, T* __restrict__ y, float* __restrict__ mean,
+                                                          float* __restrict__ rstd, int rows, float eps) {
+  pdl_trigger();
+  pdl_wait();
+  constexpr int H = VEC * 64;
+  constexpr int R = kLnFwdRows;
+  const int lane = threadIdx.x & 31;
+  const int row0 = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
+  if (row0 >= rows) return;
+  Raw2<T> raw[R][VEC];
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int row = min(row0 + r, rows - 1);  // rows past the end re-read the last row (never stored)
+    const T* xr = x + (int64_t)row * xs;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) raw[r][i] = ldraw2(xr + (i * 32 + lane) * 2);
+  }
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int row = row0 + r;
+    float2 v[VEC];
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      v[i] = cvt2(raw[r][i]);
+      s += v[i].x + v[i].y;
+    }
+    const float mu = warp_sum(s) * (1.0f / H);
+    float q = 0.f;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      const float a = v[i].x - mu, b = v[i].y - mu;
+      q += a * a + b * b;
+    }
+    const float rs = rsqrtf(warp_sum(q) * (1.0f / H) + eps);
+    if (row < rows) {
+      T* yr = y + (int64_t)row * H;
+#pragma unroll
+      for (int i = 0; i < VEC; ++i) {
+        const int c = (i * 32 + lane) * 2;
+        const float2 g = ld2f(gamma + c), bt = ld2f(beta + c);
+        st2(yr + c, make_float2((v[i].x - mu) * rs * g.x + bt.x, (v[i].y - mu) * rs * g.y + bt.y));
+      }
+      if (lane == 0) {
+        mean[row] = mu;
+        rstd[row] = rs;
+      }
+    }
+  }
+}
+
+// ln_bwd_kernel with two-element lane groups (same outputs, same partial layout ws[3][gridDim.x][H])
+template <typename T, int VEC, bool HAS_RES, bool COLSUM, bool OUT2 = false>
+__global__ void __launch_bounds__(kLnBwdWarps * 32, 2)
+    ln_bwd_pair_kernel(const T* __restrict__ dy, const T* __restrict__ x, int64_t xs, const float* __restrict__ gamma, const float* __restrict__ mean,
+                       const float* __restrict__ rstd, const T* __restrict__ dres, T* __restrict__ dx, int64_t dxs, float* __restrict__ ws, int rows,
+                       const T* __restrict__ z2 = nullptr, T* __restrict__ dx2 = nullptr, DropParams dp = DropParams{}) {
+  pdl_trigger();
+  pdl_wait();
+  constexpr int H = VEC * 64;
+  const bool dropping = OUT2 && dp.thr != 0;
+  const uint32_t dstep = dropping ? drop_step(dp) : 0u;
+  __shared__ float red[kLnBwdWarps][H];
+  const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
+  float2 gam[VEC], dg[VEC], db[VEC], dc[VEC];
+#pragma unroll
+  for (int i = 0; i < VEC; ++i) {
+    gam[i] = ld2f(gamma + (i * 32 + lane) * 2);
+    dg[i] = make_float2(0.f, 0.f);
+    db[i] = dg[i];
+    dc[i] = dg[i];
+  }
+  const int stride = gridDim.x * kLnBwdWarps;
+  int row = blockIdx.x * kLnBwdWarps + warp;
+  Raw2<T> rx[VEC], rdy[VEC], rdr[VEC];
+  float mu = 0.f, rs = 0.f;
+  const bool has_z = OUT2 && z2 != nullptr;
+  auto fetch = [&](int r) {
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      const int c = (i * 32 + lane) * 2;
+      rx[i] = ldraw2(x + (int64_t)r * xs + c);
+      rdy[i] = ldraw2(dy + (int64_t)r * H + c);
+      if (HAS_RES) rdr[i] = ldraw2(dres + (int64_t)r * H + c);
+    }
+    mu = mean[r];
+    rs = rstd[r];
+  };
+  if (row < rows) fetch(row);
+  while (row < rows) {
+    float2 xh[VEC], d[VEC], res[VEC];
+    const float cmu = mu, crs = rs;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      xh[i] = cvt2(rx[i]);
+      d[i] = cvt2(rdy[i]);
+      if (HAS_RES) res[i] = cvt2(rdr[i]);
+    }
+    const int cur = row;
+    row += stride;
+    if (row < rows) fetch(row);
+
+    float c1 = 0.f, c2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      xh[i].x = (xh[i].x - cmu) * crs;
+      xh[i].y = (xh[i].y - cmu) * crs;
+      dg[i].x += d[i].x * xh[i].x; dg[i].y += d[i].y * xh[i].y;
+      db[i].x += d[i].x; db[i].y += d[i].y;
+      d[i].x *= gam[i].x; d[i].y *= gam[i].y;
+      c1 += d[i].x + d[i].y;
+      c2 += d[i].x * xh[i].x + d[i].y * xh[i].y;
+    }
+    Raw2<T> rz[VEC];
+    if (has_z) {
+#pragma unroll
+      for (int i = 0; i < VEC; ++i) rz[i] = ldraw2(z2 + (int64_t)cur * H + (i * 32 + lane) * 2);
+    }
+    c1 = warp_sum(c1) * (1.0f / H);
+    c2 = warp_sum(c2) * (1.0f / H);
+    T* dxr = dx + (int64_t)cur * dxs;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      const int c = (i * 32 + lane) * 2;
+      float2 o;
+      o.x = crs * (d[i].x - c1 - xh[i].x * c2);
+      o.y = crs * (d[i].y - c1 - xh[i].y * c2);
+      if (HAS_RES) { o.x += res[i].x; o.y += res[i].y; }
+      st2(dxr + c, o);
+      if (OUT2) {
+        const T* tag = nullptr;
+        float2 q = make_float2(round_as(o.x, tag), round_as(o.y, tag));
+        if (dropping) drop_apply2(q, dp, dstep, (uint64_t)cur * H + c);
+        if (has_z) {
+          const float2 zz = cvt2(rz[i]);
+          q.x *= gelu_grad_f(zz.x); q.y *= gelu_grad_f(zz.y);
+        }
+        st2(dx2 + (int64_t)cur * H + c, q);
+        if (COLSUM) { dc[i].x += q.x; dc[i].y += q.y; }
+      } else if (COLSUM) {
+        dc[i].x += o.x; dc[i].y += o.y;
+      }
+    }
+  }
+  const int nparts = gridDim.x;
+#pragma unroll 1
+  for (int k = 0; k < (COLSUM ? 3 : 2); ++k) {
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) {
+      const float2 v = k == 0 ? dg[i] : (k == 1 ? db[i] : dc[i]);
+      *reinterpret_cast<float2*>(&red[warp][(i * 32 + lane) * 2]) = v;
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < H; c += blockDim.x) {
+      float s = 0.f;
+#pragma unroll
+      for (int w = 0; w < kLnBwdWarps; ++w) s += red[w][c];
+      ws[((size_t)k * nparts + blockIdx.x) * H + c] = s;
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // row-streaming kernels with per-column partial sums: GELU backward, plain column sums
 // block = (TX column groups of 4) x (TY rows); grid = (row parts, column chunks)
 // ---------------------------------------------------------------------------------------------
@@ -484,9 +674,9 @@ struct RowsGeom {
   int tx, ty, gx, gy;
 };
 static bool rows_geom(int rows, int cols, RowsGeom* g) {
-  if (cols % 128 != 0) return false;
+  if (cols % 64 != 0) return false;
   const int cg = cols / 4;
-  int tx = 32;
+  int tx = 16;  // cols % 128 == 64: half-warp rows of 16 column groups
   for (int cand : {128, 96, 64, 32})
     if (cg % cand == 0) { tx = cand; break; }
   g->tx = tx;
@@ -504,7 +694,7 @@ template <typename T>
 static int launch_rows_colsum(bool gelu, const void* a, const void* z, void* out, float* colsum,
                               void* ws, size_t ws_bytes, int rows, int cols, cudaStream_t st, const DropParams& dp = DropParams{}) {
   RowsGeom g;
-  VITB_REQUIRE(rows_geom(rows, cols, &g), "colsum: cols=%d must be a multiple of 128", cols);
+  VITB_REQUIRE(rows_geom(rows, cols, &g), "colsum: cols=%d must be a multiple of 64", cols);
   int ty8 = 0, gx8 = 0;
   if (gelu && sizeof(T) == 2 && gelu8_geom(rows, cols, &ty8, &gx8) && ((uintptr_t)a | (uintptr_t)z | (uintptr_t)out) % 16 == 0 &&
       (colsum == nullptr || (ws != nullptr && ws_bytes >= (size_t)gx8 * cols * sizeof(float)))) {
@@ -752,29 +942,34 @@ int vitb_cast_f32_to_bf16(const float* src, void* dst, int64_t n, void* stream) 
   return 0;
 }
 
-#define VITB_DISPATCH_VEC(H, ...)                                                     \
-  switch ((H) / 128) {                                                                \
-    case 1: { constexpr int VEC = 1; __VA_ARGS__; } break;                            \
-    case 2: { constexpr int VEC = 2; __VA_ARGS__; } break;                            \
-    case 3: { constexpr int VEC = 3; __VA_ARGS__; } break;                            \
-    case 4: { constexpr int VEC = 4; __VA_ARGS__; } break;                            \
-    case 6: { constexpr int VEC = 6; __VA_ARGS__; } break;                            \
-    case 8: { constexpr int VEC = 8; __VA_ARGS__; } break;                            \
-    default: ::vitb::set_error("layernorm: H=%d unsupported (128*{1,2,3,4,6,8})", H); return -1; \
+// H % 128 == 0: the four-element kernels with VEC = H / 128; H % 128 == 64: the two-element (pair) kernels with VEC = H / 64
+#define VITB_LN_CASE4(HV, STMT) case 2 * HV: { constexpr int VEC = HV; STMT; } break;
+#define VITB_LN_CASE2(HV, STMT) case HV: { constexpr int VEC = HV; STMT; } break;
+#define VITB_DISPATCH_VEC(H, QUAD, PAIR)                                                                              \
+  switch ((H) % 64 == 0 ? (H) / 64 : 0) {                                                                             \
+    VITB_LN_CASE2(1, PAIR) VITB_LN_CASE4(1, QUAD) VITB_LN_CASE2(3, PAIR) VITB_LN_CASE4(2, QUAD)                       \
+    VITB_LN_CASE2(5, PAIR) VITB_LN_CASE4(3, QUAD) VITB_LN_CASE2(7, PAIR) VITB_LN_CASE4(4, QUAD)                       \
+    VITB_LN_CASE2(9, PAIR) VITB_LN_CASE4(5, QUAD) VITB_LN_CASE2(11, PAIR) VITB_LN_CASE4(6, QUAD)                      \
+    VITB_LN_CASE2(13, PAIR) VITB_LN_CASE4(7, QUAD) VITB_LN_CASE2(15, PAIR) VITB_LN_CASE4(8, QUAD)                     \
+    default: ::vitb::set_error("layernorm: H=%d unsupported (a multiple of 64 up to 1024)", H); return -1;            \
   }
 
 int vitb_layernorm_fwd(const void* x, int64_t xs, const float* gamma, const float* beta, void* y,
                        float* mean, float* rstd, int rows, int H, float eps, int dt, void* stream) {
   VITB_REQUIRE(x && gamma && beta && y && mean && rstd, "layernorm_fwd: null pointer");
-  VITB_REQUIRE(rows >= 0 && H % 128 == 0 && xs % 4 == 0, "layernorm_fwd: bad shape rows=%d H=%d stride=%lld", rows, H, (long long)xs);
+  VITB_REQUIRE(rows >= 0 && H % 64 == 0 && xs % 4 == 0, "layernorm_fwd: bad shape rows=%d H=%d stride=%lld", rows, H, (long long)xs);
   if (rows == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = ceil_div(rows, 8 * kLnFwdRows);
+#define VITB_LN_FWD(T)                                                                                                         \
+  VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_fwd_kernel<T, VEC>), blocks, 256, 0, st, (const T*)x, xs, gamma, beta, (T*)y, mean, rstd, rows, eps)), \
+                    (VITB_LAUNCH((ln_fwd_pair_kernel<T, VEC>), blocks, 256, 0, st, (const T*)x, xs, gamma, beta, (T*)y, mean, rstd, rows, eps)))
   if (dt == VITB_BF16) {
-    VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_fwd_kernel<bf16, VEC>), blocks, 256, 0, st, (const bf16*)x, xs, gamma, beta, (bf16*)y, mean, rstd, rows, eps)));
+    VITB_LN_FWD(bf16);
   } else {
-    VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_fwd_kernel<float, VEC>), blocks, 256, 0, st, (const float*)x, xs, gamma, beta, (float*)y, mean, rstd, rows, eps)));
+    VITB_LN_FWD(float);
   }
+#undef VITB_LN_FWD
   VITB_LAUNCH_OK();
   return 0;
 }
@@ -788,7 +983,7 @@ int vitb_layernorm_bwd_fused(const void* dy, const void* x, int64_t xs, const fl
                              float* dx2_colsum, const vitb_dropout_t* drop, void* ws, size_t ws_bytes, int rows, int H, int dt,
                              void* stream) {
   VITB_REQUIRE(dy && x && gamma && mean && rstd && dres && dx && dgamma && dbeta && dx2 && dx2_colsum && ws, "layernorm_bwd_fused: null pointer");
-  VITB_REQUIRE(rows > 0 && H % 128 == 0 && xs % 4 == 0 && dxs % 4 == 0, "layernorm_bwd_fused: bad shape");
+  VITB_REQUIRE(rows > 0 && H % 64 == 0 && xs % 4 == 0 && dxs % 4 == 0, "layernorm_bwd_fused: bad shape");
   VITB_REQUIRE(ws_bytes >= vitb_layernorm_bwd_ws_bytes(rows, H), "layernorm_bwd_fused: workspace too small");
   VITB_REQUIRE(dx2 != dx && dx2 != dy && dx2 != dres, "layernorm_bwd_fused: dx2 must not alias another operand");
   DropParams dp;
@@ -796,13 +991,17 @@ int vitb_layernorm_bwd_fused(const void* dy, const void* x, int64_t xs, const fl
   if (void* d = defer_alloc(vitb_layernorm_bwd_ws_bytes(rows, H))) ws = d;  // deferred second pass: the partials must outlive this call
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = ln_bwd_blocks(rows);
+#define VITB_LN_BWD_FUSED(T)                                                                                                      \
+  VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_bwd_kernel<T, VEC, true, true, true>), blocks, kLnBwdWarps * 32, 0, st, (const T*)dy, (const T*)x, xs, gamma, \
+                                    mean, rstd, (const T*)dres, (T*)dx, dxs, (float*)ws, rows, (const T*)z, (T*)dx2, dp)),                          \
+                    (VITB_LAUNCH((ln_bwd_pair_kernel<T, VEC, true, true, true>), blocks, kLnBwdWarps * 32, 0, st, (const T*)dy, (const T*)x, xs,     \
+                                 gamma, mean, rstd, (const T*)dres, (T*)dx, dxs, (float*)ws, rows, (const T*)z, (T*)dx2, dp)))
   if (dt == VITB_BF16) {
-    VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_bwd_kernel<bf16, VEC, true, true, true>), blocks, kLnBwdWarps * 32, 0, st, (const bf16*)dy, (const bf16*)x, xs,
-                                      gamma, mean, rstd, (const bf16*)dres, (bf16*)dx, dxs, (float*)ws, rows, (const bf16*)z, (bf16*)dx2, dp)));
+    VITB_LN_BWD_FUSED(bf16);
   } else {
-    VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_bwd_kernel<float, VEC, true, true, true>), blocks, kLnBwdWarps * 32, 0, st, (const float*)dy, (const float*)x,
-                                      xs, gamma, mean, rstd, (const float*)dres, (float*)dx, dxs, (float*)ws, rows, (const float*)z, (float*)dx2, dp)));
+    VITB_LN_BWD_FUSED(float);
   }
+#undef VITB_LN_BWD_FUSED
   VITB_LAUNCH_OK();
   VITB_CUDA_OK(::vitb::launch_finalize((const float*)ws, blocks, H, dgamma, dbeta, dx2_colsum, 3, st));
   return 0;
@@ -813,7 +1012,7 @@ int vitb_layernorm_bwd(const void* dy, const void* x, int64_t xs, const float* g
                        float* dbeta, float* dx_colsum, void* ws, size_t ws_bytes, int rows, int H, int dt,
                        void* stream) {
   VITB_REQUIRE(dy && x && gamma && mean && rstd && dx && dgamma && dbeta && ws, "layernorm_bwd: null pointer");
-  VITB_REQUIRE(rows > 0 && H % 128 == 0 && xs % 4 == 0 && dxs % 4 == 0, "layernorm_bwd: bad shape");
+  VITB_REQUIRE(rows > 0 && H % 64 == 0 && xs % 4 == 0 && dxs % 4 == 0, "layernorm_bwd: bad shape");
   VITB_REQUIRE(ws_bytes >= vitb_layernorm_bwd_ws_bytes(rows, H), "layernorm_bwd: workspace too small");
   if (void* d = defer_alloc(vitb_layernorm_bwd_ws_bytes(rows, H))) ws = d;  // deferred second pass: the partials must outlive this call
   cudaStream_t st = (cudaStream_t)stream;
@@ -821,7 +1020,9 @@ int vitb_layernorm_bwd(const void* dy, const void* x, int64_t xs, const float* g
   const bool res = dres != nullptr, cs = dx_colsum != nullptr;
 #define VITB_LN_BWD(T, RES, CS)                                                                                              \
   VITB_DISPATCH_VEC(H, (VITB_LAUNCH((ln_bwd_kernel<T, VEC, RES, CS>), blocks, kLnBwdWarps * 32, 0, st, (const T*)dy, (const T*)x, xs, gamma, mean, rstd, \
-                                                                                         (const T*)dres, (T*)dx, dxs, (float*)ws, rows, nullptr, nullptr, DropParams{})))
+                                                                                         (const T*)dres, (T*)dx, dxs, (float*)ws, rows, nullptr, nullptr, DropParams{})), \
+                    (VITB_LAUNCH((ln_bwd_pair_kernel<T, VEC, RES, CS>), blocks, kLnBwdWarps * 32, 0, st, (const T*)dy, (const T*)x, xs, gamma, mean, rstd, \
+                                 (const T*)dres, (T*)dx, dxs, (float*)ws, rows, nullptr, nullptr, DropParams{})))
   if (dt == VITB_BF16) {
     if (res && cs) { VITB_LN_BWD(bf16, true, true); } else if (res) { VITB_LN_BWD(bf16, true, false); }
     else if (cs) { VITB_LN_BWD(bf16, false, true); } else { VITB_LN_BWD(bf16, false, false); }

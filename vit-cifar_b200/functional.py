@@ -49,14 +49,16 @@ class Dims:
         return 1.0 / (self.H ** 0.5)
 
     def check(self) -> None:
-        if self.H % 128 != 0:
-            raise ValueError(f"hidden={self.H} must be a multiple of 128 for the vectorised LayerNorm kernels")
+        # widths of 64 mod 128 run the LayerNorm kernels with two-element lane groups and the GEMMs with a partial last
+        # 128-column tile; 1024 is the widest LayerNorm row one warp holds in registers
+        if self.H % 64 != 0 or not 64 <= self.H <= 1024:
+            raise ValueError(f"hidden={self.H} must be a multiple of 64 in [64, 1024] for the vectorised LayerNorm kernels")
         if self.H % self.heads != 0 or self.d not in (32, 64):
             raise ValueError(f"head_dim={self.H}/{self.heads} must be 32 or 64 for the fused attention kernel")
         if self.T > 128:
             raise ValueError(f"{self.T} tokens > 128: the fused short-sequence attention kernel keeps (T x T) on chip")
-        if self.use_mlp and self.M % 128 != 0:
-            raise ValueError(f"mlp_hidden={self.M} must be a multiple of 128")
+        if self.use_mlp and (self.M % 64 != 0 or self.M <= 0):
+            raise ValueError(f"mlp_hidden={self.M} must be a positive multiple of 64")
 
 
 class SideStream:
