@@ -117,7 +117,8 @@ int vitb_gemm_wgrad_dbias(const void* dy, const void* x, float* dw, float* dbias
  * columns h*d..h*d+d-1 of each third;  o act (B,T,H) (= attn.flatten(2), layers.py:102)
  * lse fp32 (B,heads,T): log-sum-exp of the scaled scores (saved instead of the (B,h,T,T) map).
  * attn_map fp32 (B,heads,T,T) or NULL: the softmax map itself (save_attn_map, layers.py:99-100).
- * scale = 1/sqrt(features) (layers.py:79,97).  d in {32,64}, T <= 128. */
+ * scale = 1/sqrt(features) (layers.py:79,97).  T <= 128, d in {32,64,96,128}; fp32: staged tiles <= 227 KB
+ * (3·T·d + T·T floats forward, 4·T·d + 2·T·T backward; checked for d = 96 / 128). */
 int vitb_attn_fwd(const void* qkv, void* o, float* lse, float* attn_map, int B, int T, int heads,
                   int d, float scale, int dt, void* stream);
 /* dqkv act (B,T,3H) from d_o act (B,T,H): dP = dO·Vᵀ; dS = P∘(dP − D), D_i = rowsum(P∘dP)_i = sum_d dO_id·O_id;

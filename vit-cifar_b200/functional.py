@@ -53,8 +53,9 @@ class Dims:
         # 128-column tile; 1024 is the widest LayerNorm row one warp holds in registers
         if self.H % 64 != 0 or not 64 <= self.H <= 1024:
             raise ValueError(f"hidden={self.H} must be a multiple of 64 in [64, 1024] for the vectorised LayerNorm kernels")
-        if self.H % self.heads != 0 or self.d not in (32, 64):
-            raise ValueError(f"head_dim={self.H}/{self.heads} must be 32 or 64 for the fused attention kernel")
+        # 96 and 128 run as three 32-column / two 64-column panels of the 32 / 64 attention tiles
+        if self.H % self.heads != 0 or self.d not in (32, 64, 96, 128):
+            raise ValueError(f"head_dim={self.H}/{self.heads} must be 32, 64, 96 or 128 for the fused attention kernel")
         if self.T > 128:
             raise ValueError(f"{self.T} tokens > 128: the fused short-sequence attention kernel keeps (T x T) on chip")
         if self.use_mlp and (self.M % 64 != 0 or self.M <= 0):
